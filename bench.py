@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark: Atlas (floating base, nv = 36) forward-dynamics evaluations per second.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dtype f32|f64]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dtype f32|f64] [--dump-outputs DIR]
 
 Workload (BASELINE.json metric, SURVEY 8(d) "Headline"): Atlas v5 with a QuaternionFloating root (nq 37, nv 36, 31 bodies),
 `dynamics!` with joint torques, fp32, batch 2^20 per GPU.  A "step" is one pass of the forward-dynamics kernel over the whole
@@ -14,6 +14,12 @@ One JSON line on stdout (rank 0).  `value` = evaluations/s with inputs resident 
 `cpu_baseline` = the CPU oracle (port of the reference's CRBA + RNEA + Cholesky path) on a bounded sample.
 
 `--impl reference` times that CPU path alone (the reference itself is Julia and cannot run here; see DESIGN.md).
+
+`--dump-outputs DIR` writes what the last timed step computed, v̇ of rank 0, as DIR/vd.npy ([36, n], the run's dtype): the whole
+batch when it fits in 48 MB, else the same seeded sample of n columns in every run with the same arguments.  The inputs depend on
+the arguments alone, so two builds can be compared output for output.
+
+Nothing is written into the source tree: cubins compiled at run time go to a temporary copy of the build's cubin cache.
 """
 from __future__ import annotations
 
@@ -29,8 +35,10 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 
 BYTES_PER_EVAL = {"f32": 580, "f64": 1160}      # (37 + 36 + 36 in, 36 out) scalars, BASELINE.md section 4
+DUMP_BYTES = 48 << 20
 METRIC = "ABA evals/sec for Atlas 30-DoF at batch 2^20; achieved HBM GB/s vs peak"
 
 
@@ -306,6 +314,34 @@ def other_configs(steps):
     return out
 
 
+def private_jit_cache():
+    """Point the cubin cache at a temporary copy of the one build() filled (csrc/jit_cache), so that kernels compiled during the run
+    never land in the source tree, which may be read-only.  Returns the TemporaryDirectory (removed when it is closed)."""
+    import shutil
+    import tempfile
+    if os.environ.get("RBD_JIT_CACHE"):
+        return None
+    tmp = tempfile.TemporaryDirectory(prefix="rbd_jit_cache_")
+    src = os.path.join(ROOT, "rigidbodydynamics", "jl_b200", "csrc", "jit_cache")
+    if os.path.isdir(src):
+        for f in os.listdir(src):
+            if f.endswith(".cubin"):
+                shutil.copyfile(os.path.join(src, f), os.path.join(tmp.name, f))
+    os.environ["RBD_JIT_CACHE"] = tmp.name
+    return tmp
+
+
+def output_sample(vd):
+    """Device copy of what --dump-outputs writes: v̇ [rows, B], or above DUMP_BYTES a fixed seeded sample of its columns."""
+    import torch
+    rows, B = vd.shape
+    n = min(B, DUMP_BYTES // (rows * vd.element_size()))
+    if n == B:
+        return vd.clone()
+    idx = np.sort(np.random.Generator(np.random.PCG64(0)).choice(B, n, replace=False))
+    return vd[:, torch.from_numpy(idx).to(vd.device)]
+
+
 def add_rooflines(cfgs, peak):
     """Per-config roofline objects (HBM, algorithmic bytes) next to the raw rates; ncu summaries of the kernels behind them are under
     profiles/r2_*_summary.txt (dram__bytes_read/write, issue-active, stall reasons)."""
@@ -487,10 +523,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-config5", action="store_true", help="N > 1: skip BASELINE config 5 (2^22 samples in total, result gather timed)")
     ap.add_argument("--no-other", action="store_true", help="skip the secondary configs (fp64, RNEA, CRBA, ext. wrenches)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write v̇ of the last timed step to DIR/vd.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl ours")
         return run_reference(args)
+    jit_cache = private_jit_cache()
 
     import torch
     import rigidbodydynamics.jl_b200 as rbd
@@ -538,6 +578,7 @@ def main():
     barrier()
     t_wall1 = time.time()
     ms = ev0.elapsed_time(ev1)
+    dump = output_sample(result.vd) if args.dump_outputs and rank == 0 else None
     # keep the GPU under the same load until the sampler has a few readings inside a loaded window
     t_load_end = t_wall1
     if sampler and (t_wall1 - t_wall0) < 0.6:
@@ -659,8 +700,13 @@ def main():
             scale = np.maximum(1.0, np.abs(ref).max(0))
             out["accuracy"] = {"max_rel_err_vs_fp64_oracle": float((np.abs(got - ref).max(0) / scale).max()), "samples": n}
         _emit(out)
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "vd.npy"), dump.cpu().numpy())
     if dist is not None:
         dist.destroy_process_group()
+    if jit_cache is not None:
+        jit_cache.cleanup()
 
 
 if __name__ == "__main__":

@@ -197,7 +197,7 @@ class SpecProgram:
         self.desc, self.algo, self.dtype = desc, algo, np.dtype(dtype)
         src, self.stats = spec_source(desc, algo, dtype, has_in2, has_out1, 0)
         tag = hashlib.sha1(src.encode()).hexdigest()[:16]
-        d = os.path.join(tempfile.gettempdir(), "rbd_spec_cpu")
+        d = os.path.join(tempfile.gettempdir(), f"rbd_spec_cpu_{os.getuid()}")      # per user: /tmp is shared
         os.makedirs(d, exist_ok=True)
         so = os.path.join(d, f"spec_{tag}.so")
         if not os.path.exists(so):

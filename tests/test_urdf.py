@@ -6,7 +6,7 @@ import pytest
 
 import rigidbodydynamics.jl_b200 as rbd
 from oracle import Oracle
-from tests.util import REF_URDF, have_reference, rand_inputs
+from tests.util import GOLD, rand_inputs
 
 ATLAS_ORDER = ["pelvis_to_world", "back_bkz", "l_leg_hpz", "r_leg_hpz", "back_bky", "l_leg_hpx", "r_leg_hpx", "back_bkx",
                "l_leg_hpy", "r_leg_hpy", "l_arm_shz", "neck_ay", "r_arm_shz", "l_leg_kny", "r_leg_kny", "l_arm_shx",
@@ -37,22 +37,23 @@ def test_atlas_joint_order_and_sizes():
     assert fixed.joint_names == ATLAS_ORDER[1:]
 
 
-@pytest.mark.skipif(not have_reference(), reason="reference URDF fixtures not present on this machine")
 @pytest.mark.parametrize("name", ["atlas", "valkyrie"])
 def test_json_description_equals_reference_urdf(name):
+    """The JSON description gives the mechanism parse_urdf built from the reference's test/urdf/<name>.urdf (stored flattened in
+    tests/golden/reference_urdf.npz by tools/make_fixtures.py)."""
+    ref = np.load(os.path.join(GOLD, "reference_urdf.npz"))
     for floating in (False, True):
         a = rbd.load_model(name, floating=floating).flatten()
-        b = rbd.parse_urdf(os.path.join(REF_URDF, name + ".urdf"), floating=floating).flatten()
-        assert a.joint_names == b.joint_names
+        key = f"{name}_{'floating' if floating else 'fixed'}"
+        assert a.joint_names == ref[key + "_joint_names"].tolist()
         for f in ("parent", "jtype", "X_tree", "jparam", "inertia"):
-            assert np.array_equal(getattr(a, f), getattr(b, f)), f
+            assert np.array_equal(getattr(a, f), ref[f"{key}_{f}"]), f
 
 
-@pytest.mark.skipif(not have_reference(), reason="reference URDF fixtures not present on this machine")
 def test_reference_small_urdfs_parse():
-    acro = rbd.parse_urdf(os.path.join(REF_URDF, "Acrobot.urdf"))
+    acro = rbd.parse_urdf(os.path.join(GOLD, "urdf", "Acrobot.urdf"))
     assert (acro.num_positions(), acro.num_velocities()) == (2, 2)
-    slider = rbd.parse_urdf(os.path.join(REF_URDF, "planar_slider.urdf"))
+    slider = rbd.parse_urdf(os.path.join(GOLD, "urdf", "planar_slider.urdf"))
     assert all(isinstance(j.joint_type, rbd.Planar) for j in slider.joints)
 
 

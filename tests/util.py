@@ -5,7 +5,7 @@ import numpy as np
 
 import rigidbodydynamics.jl_b200 as rbd
 
-REF_URDF = "/root/reference/test/urdf"
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 ALL_JOINT_TYPES = ([rbd.QuaternionFloating] + [rbd.Revolute] * 5 + [rbd.Fixed] * 5 + [rbd.Prismatic] * 5
                    + [rbd.Planar] * 5 + [rbd.SPQuatFloating] * 2 + [rbd.SinCosRevolute] * 2
                    + [rbd.QuaternionSpherical] * 2)
@@ -46,10 +46,6 @@ def rel_err(got, ref):
     """max over the batch of |got - ref|_inf / max(1, |ref|_inf)   (SURVEY 8(d) 'Accuracy')."""
     got, ref = np.asarray(got, float), np.asarray(ref, float)
     return float((np.abs(got - ref).max(0) / np.maximum(1.0, np.abs(ref).max(0))).max())
-
-
-def have_reference():
-    return os.path.isdir(REF_URDF)
 
 
 def make_duals(mech, q, v, tau, seed):
