@@ -50,7 +50,9 @@ int fail_cuda(cudaError_t e, const char* what) {
 }
 #define CUDA_TRY(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) return fail_cuda(e_, #expr); } while (0)
 
-struct DeviceProps { int dev = 0; int sms = 0; int max_smem_optin = 0; int smem_per_sm = 0; bool ok = false; };
+}  // namespace
+
+namespace rbd {
 int get_props(DeviceProps& p) {
   static std::mutex mu;
   static DeviceProps cache[64];
@@ -75,6 +77,35 @@ int get_props(DeviceProps& p) {
   p = q;
   return RBD_OK;
 }
+
+int configure_once(const void* kernel, const DeviceProps& p) {
+  static std::mutex mu;
+  static std::set<std::pair<const void*, int>> done;
+  std::lock_guard<std::mutex> lk(mu);
+  if (done.count({kernel, p.dev})) return RBD_OK;
+  cudaFuncAttributes fa{};
+  CUDA_TRY(cudaFuncGetAttributes(&fa, kernel));
+  CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, p.max_smem_optin - (int)fa.sharedSizeBytes));
+  CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  done.insert({kernel, p.dev});
+  return RBD_OK;
+}
+
+// The pair gives the Tensor-Memory CTA room in the register file (65536 per SM) by running fewer shared-memory blocks: small
+// models are not limited by shared memory, and persistent shared-memory blocks would keep the CTA off the SM until they drain
+// the queue.  It only pays when shared memory (not the register file) limits the single kernel's residency, i.e. when the pair
+// puts at least 15 % more warps on the SM, and when the batch has enough groups to keep both kernels' warps busy.
+int pair_blocks(int sms, int bps, int regs_smem, int regs_tmem, int tm_warps, int64_t ngroups) {
+  const int rs = ((regs_smem + 7) / 8) * 8 * 32, rt = ((regs_tmem + 7) / 8) * 8 * 32 * tm_warps;
+  if (rt + rs > 65536) return 0;
+  const int with_pair = std::max(1, std::min(bps, (65536 - rt) / rs));
+  if ((with_pair + tm_warps) * 100 < bps * 115) return 0;
+  if (ngroups < (int64_t)(with_pair + tm_warps / 2) * sms) return 0;
+  return with_pair;
+}
+}  // namespace rbd
+
+namespace {
 
 template <class T> const ModelDev<T>& dev_model(const HostModel& m);
 template <> const ModelDev<float>& dev_model<float>(const HostModel& m) { return m.dev32; }
@@ -416,20 +447,6 @@ __global__ void __launch_bounds__(NT, sizeof(T) == 4 ? 28 : 12) kin_kernel(const
   }
 }
 
-// Opt a kernel into large dynamic shared memory ONCE per (kernel, device): the attribute is process-global per kernel, so
-// setting it to each call's exact size would race between host threads using different model handles.
-int configure_once(const void* kernel, const DeviceProps& p) {
-  static std::mutex mu;
-  static std::set<std::pair<const void*, int>> done;
-  std::lock_guard<std::mutex> lk(mu);
-  if (done.count({kernel, p.dev})) return RBD_OK;
-  cudaFuncAttributes fa{};
-  CUDA_TRY(cudaFuncGetAttributes(&fa, kernel));
-  CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, p.max_smem_optin - (int)fa.sharedSizeBytes));
-  CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  done.insert({kernel, p.dev});
-  return RBD_OK;
-}
 template <class T> struct BodiesArgs {
   const T* q; const T* v; const T* vd; const T* wext;
   T* acc; T* jw;
@@ -493,38 +510,28 @@ template <class K> int configure(K kernel, int nt, size_t smem, const DeviceProp
   return RBD_OK;
 }
 
-template <class T> struct AbaArgs; template <class T> struct RneaArgs; template <class T> struct CrbaArgs;
-template <class T> void set_scratch(AbaArgs<T>& a, T* s);
-template <class T> void set_scratch(RneaArgs<T>& a, T* s);
-template <class T> void set_scratch(CrbaArgs<T>&, T*);
-
-// Launch `kernel` persistently (blocks_per_SM x SMs blocks looping over groups of NT samples).  `scratch_rows` > 0
-// requests a stream-ordered scratch of that many rows per resident thread (the external-wrench path).
-template <class T, class Kern, class Args>
-int launch(Kern kernel, const ModelDev<T>& M, Args a, int nt, int rows, int scratch_rows, cudaStream_t stream) {
+// Launch `kernel(args...)` persistently: blocks_per_SM x SMs blocks of `nt` threads (fewer for a small batch) loop over the
+// groups of `nt` of the `work` items, with `rows` stash rows of T per thread in shared memory.  `scratch_rows` > 0 requests a
+// stream-ordered scratch of that many rows per resident thread (external wrenches, momentum-matrix poses): it is stored into
+// `*scratch`, a field of one of `args`, before the launch.
+template <class T, class Kern, class... Args>
+int launch(Kern kernel, int nt, int rows, int64_t work, T** scratch, int scratch_rows, cudaStream_t stream, const Args&... args) {
   DeviceProps p;
   if (int rc = get_props(p)) return rc;
   const size_t smem = (size_t)rows * nt * sizeof(T);
   int bps = 0;
   if (int rc = configure(kernel, nt, smem, p, bps)) return rc;
-  const int64_t ngroups = (a.B + nt - 1) / nt;
+  const int64_t ngroups = (work + nt - 1) / nt;
   const int grid = (int)std::min<int64_t>(ngroups, (int64_t)bps * p.sms);
-  void* scratch = nullptr;
-  if (scratch_rows > 0) {
-    CUDA_TRY(cudaMallocAsync(&scratch, (size_t)scratch_rows * grid * nt * sizeof(T), stream));
-    set_scratch(a, (T*)scratch);
-  }
-  kernel<<<grid, nt, smem, stream>>>(M, a);
+  if (scratch_rows > 0) CUDA_TRY(cudaMallocAsync((void**)scratch, (size_t)scratch_rows * grid * nt * sizeof(T), stream));
+  kernel<<<grid, nt, smem, stream>>>(args...);
   cudaError_t e = cudaGetLastError();
-  if (scratch) cudaFreeAsync(scratch, stream);
+  if (scratch_rows > 0) cudaFreeAsync(*scratch, stream);
   if (e != cudaSuccess) return fail_cuda(e, "kernel launch");
   g_launch.kernels_launched += 1;
   g_launch.grid = grid; g_launch.block = nt; g_launch.smem_bytes = (int)smem; g_launch.blocks_per_sm = bps;
   return RBD_OK;
 }
-template <class T> void set_scratch(AbaArgs<T>& a, T* s) { a.scratch = s; }
-template <class T> void set_scratch(RneaArgs<T>& a, T* s) { a.scratch = s; }
-template <class T> void set_scratch(CrbaArgs<T>&, T*) {}
 
 constexpr int kNT = 32;   // threads per block: one warp; warps never synchronise with each other
 
@@ -532,21 +539,13 @@ constexpr int kNT = 32;   // threads per block: one warp; warps never synchronis
 // side stream, both claiming groups of 32 samples from one atomic counter.  fp32: one stash row = one TMEM column, so the 512
 // columns hold the stash of 8 warps (two column halves x four lane quadrants); fp64: two columns per row, 4 warps.  On Atlas
 // that is 8 + 8 resident warps/SM in fp32 (16 x 32 x 128 registers = the whole register file) and 4 + 4 in fp64.
-// `used` = false (and nothing launched) when the batch is too small to feed both kernels or RBD_NO_TMEM is set.
-// Which entry points use the kernel pair by default (RBD_DUO_RNEA=0/1, RBD_DUO_EXT=0/1 override).
-constexpr bool kDuoRneaDefault = true, kDuoExtDefault = true;
-inline bool duo_enabled(const char* env, bool dflt) {
-  const char* e = getenv(env);
-  return e ? (e[0] != '0') : dflt;
-}
-
+// `used` = false (and nothing launched) when pair_blocks declines the pair or RBD_NO_TMEM is set.
 template <class T, class KS, class KT, class Args>
 int launch_duo(const rbd_model* model, KS ks, KT kt, int tm_warps, const ModelDev<T>& M, Args a, int rows, int scratch_rows,
                cudaStream_t stream, bool& used) {
   used = false;
-  static const bool no_tmem = getenv("RBD_NO_TMEM") != nullptr;
-  static const int smem_blocks = getenv("RBD_SMEM_BLOCKS") ? atoi(getenv("RBD_SMEM_BLOCKS")) : 0;
-  if (no_tmem) return RBD_OK;
+  const LaunchEnv& ev = launch_env();
+  if (ev.no_tmem) return RBD_OK;
   DeviceProps p;
   if (int rc = get_props(p)) return rc;
   const int64_t ngroups = (a.B + kNT - 1) / kNT;
@@ -554,21 +553,11 @@ int launch_duo(const rbd_model* model, KS ks, KT kt, int tm_warps, const ModelDe
   int bps = 0;
   if (int rc = configure(ks, kNT, smem, p, bps)) return rc;
   if (int rc = configure_once((const void*)kt, p)) return rc;
-  {
-    // leave room in the register file for the Tensor-Memory CTA: small models are not limited by shared memory and the
-    // persistent shared-memory blocks would otherwise keep that CTA off the SM until they drain the queue
-    cudaFuncAttributes fs{}, ft{};
-    CUDA_TRY(cudaFuncGetAttributes(&fs, ks));
-    CUDA_TRY(cudaFuncGetAttributes(&ft, kt));
-    const int rs = ((fs.numRegs + 7) / 8) * 8 * kNT, rt = ((ft.numRegs + 7) / 8) * 8 * 32 * tm_warps;
-    const int with_pair = std::max(1, std::min(bps, (65536 - rt) / rs));
-    // The pair only pays when shared memory (not the register file) limits the single kernel's residency: small models
-    // already fill the SM with shared-memory blocks and are faster on the single-kernel path.
-    if ((with_pair + tm_warps) * 100 < bps * 115) return RBD_OK;
-    bps = with_pair;
-  }
-  if (smem_blocks > 0) bps = std::max(1, std::min(bps, smem_blocks));
-  if (ngroups < (int64_t)(bps + tm_warps / 2) * p.sms) return RBD_OK;     // not enough work to keep both kernels' warps busy
+  cudaFuncAttributes fs{}, ft{};
+  CUDA_TRY(cudaFuncGetAttributes(&fs, ks));
+  CUDA_TRY(cudaFuncGetAttributes(&ft, kt));
+  bps = pair_blocks(p.sms, bps, fs.numRegs, ft.numRegs, tm_warps, ngroups);
+  if (bps == 0) return RBD_OK;
   rbd_model* mm = const_cast<rbd_model*>(model);
   PairCtx ctx;      // side stream, fork / join events and a zeroed queue counter, all cached in the handle
   CUDA_TRY(pair_begin(mm, stream, ctx));
@@ -586,9 +575,8 @@ int launch_duo(const rbd_model* model, KS ks, KT kt, int tm_warps, const ModelDe
   CUDA_TRY(cudaStreamWaitEvent(side, fork, 0));
   // (profiling aid: under ncu kernels are serialised and the first one drains the queue; RBD_ONLY=smem|tmem launches
   //  just one of the two so each can be captured doing the whole batch)
-  static const char* const only = getenv("RBD_ONLY");
-  if (!only || only[0] == 's') ks<<<bps * p.sms, kNT, smem, stream>>>(M, a);
-  if (!only || only[0] == 't') kt<<<p.sms, 32 * tm_warps, 0, side>>>(M, a);
+  if (!ev.only || ev.only[0] == 's') ks<<<bps * p.sms, kNT, smem, stream>>>(M, a);
+  if (!ev.only || ev.only[0] == 't') kt<<<p.sms, 32 * tm_warps, 0, side>>>(M, a);
   cudaError_t e = cudaGetLastError();
   cudaEventRecord(join, side);
   cudaStreamWaitEvent(stream, join, 0);
@@ -600,53 +588,59 @@ int launch_duo(const rbd_model* model, KS ks, KT kt, int tm_warps, const ModelDe
   return RBD_OK;
 }
 
+// The model-specialised kernels for `key` (rbd_spec.cpp: straight-line code generated for this mechanism) when they can serve
+// the call, else `generic(nullptr)`.  fp32 specialised programs have no slow sin / cos path: if any sample met an angle beyond
+// 1e4 rad they raise a flag on the device, and `generic(gate)` enqueued behind them redoes the batch with the library path (it
+// exits at once while the flag is down).  Launch info then describes the specialised launch and counts the kernels of both.
+template <class Generic>
+int spec_or_generic(const rbd_model* model, const SpecKey& key, const SpecLaunchArgs& sa, cudaStream_t stream, Generic generic) {
+  bool used = false;
+  const int* gate = nullptr;
+  if (int rc = spec_try_launch(const_cast<rbd_model*>(model), key, sa, stream, used, g_launch, &gate)) return rc;
+  if (!used) return generic(nullptr);
+  g_launch.specialised = 1;
+  if (!gate) return RBD_OK;
+  const rbd_launch_info keep = g_launch;
+  const int rc = generic(gate);
+  const int n = g_launch.kernels_launched;
+  g_launch = keep;
+  g_launch.kernels_launched = n;
+  return rc;
+}
+
+// The generic ABA kernel for this model: multi-DoF joints below the root (GENERAL), prismatic / fixed joints (all 1-DoF kinds)
+// or revolute joints only (KINDS = 0).
+template <class T>
+int launch_generic_aba(const HostModel& hm, AbaArgs<T> a, bool ext, cudaStream_t stream) {
+  const ModelDev<T>& M = dev_model<T>(hm);
+  auto kernel = hm.general       ? (ext ? aba_kernel<T, kNT, true, true, kAllKinds> : aba_kernel<T, kNT, true, false, kAllKinds>)
+                : hm.other_kinds ? (ext ? aba_kernel<T, kNT, false, true, kAllKinds> : aba_kernel<T, kNT, false, false, kAllKinds>)
+                                 : (ext ? aba_kernel<T, kNT, false, true, 0> : aba_kernel<T, kNT, false, false, 0>);
+  return launch<T>(kernel, kNT, M.nrows, a.B, &a.scratch, ext ? 6 * hm.nb : 0, stream, M, a);
+}
+
 template <class T>
 int dynamics_t(const rbd_model* model, int64_t B, int64_t ld, const void* q, const void* v, const void* tau,
                const void* wext, void* vd, void* qd, cudaStream_t stream) {
   const HostModel& hm = model->hm;
   const ModelDev<T>& M = dev_model<T>(hm);
   AbaArgs<T> a{(const T*)q, (const T*)v, (const T*)tau, (const T*)wext, (T*)vd, (T*)qd, nullptr, ld, B};
-  const int rows = M.nrows;
-  const int sr = wext ? 6 * hm.nb : 0;
-  bool other_kinds = false;          // prismatic / fixed joints anywhere -> kernels with those code paths
-  for (int i = 0; i < hm.nb; ++i) other_kinds |= (M.body[i].kind == K_PRIS || M.body[i].kind == K_FIXED);
-#define RBD_ABA(G, E, K) launch<T>(aba_kernel<T, kNT, G, E, K>, M, a, kNT, rows, sr, stream)
-  if (!wext) {      // model-specialised kernels (rbd_spec.cpp): straight-line code generated for this mechanism
-    SpecKey key; key.algo = SPEC_ABA; key.f64 = sizeof(T) == 8; key.has_in2 = tau != nullptr; key.has_out1 = qd != nullptr;
-    const SpecLaunchArgs sa{q, v, tau, vd, qd, ld, B};
-    bool used = false;
-    std::string err;
-    const int* gate = nullptr;
-    if (int rc = spec_try_launch(const_cast<rbd_model*>(model), key, sa, stream, used, g_launch, &gate, err)) return fail(rc, err);
-    if (used) {
-      g_launch.specialised = 1;
-      if (!gate) return RBD_OK;
-      // fp32: the specialised program has no slow sin / cos path; if any sample met an angle beyond 1e4 rad (flag raised on the
-      // device) this generic launch redoes the batch with the library path, otherwise it exits at once
-      const rbd_launch_info keep = g_launch;
-      a.gate = gate;
-      const int rc = hm.general ? RBD_ABA(true, false, kAllKinds) : (other_kinds ? RBD_ABA(false, false, kAllKinds) : RBD_ABA(false, false, 0));
-      const int n = g_launch.kernels_launched;
-      g_launch = keep;
-      g_launch.kernels_launched = n;
-      return rc;
+  auto generic = [&](const int* gate) {
+    a.gate = gate;
+    if (!gate && !hm.general && !hm.other_kinds && M.nrows <= 256) {
+      // default path for all-revolute trees whose stash fits Tensor Memory (see launch_duo); its kernels take no gate
+      constexpr int kTmWarps = sizeof(T) == 4 ? 8 : 4;
+      bool used = false;
+      const int rc = launch_duo<T>(model, wext ? aba_kernel_smem_q<T, 0, true> : aba_kernel_smem_q<T, 0, false>,
+                                   wext ? aba_kernel_tmem_q<T, 512, 0, kTmWarps, true> : aba_kernel_tmem_q<T, 512, 0, kTmWarps, false>,
+                                   kTmWarps, M, a, M.nrows, wext ? 6 * hm.nb : 0, stream, used);
+      if (rc || used) return rc;
     }
-  }
-  if (!hm.general && !other_kinds && rows <= 256 && (!wext || duo_enabled("RBD_DUO_EXT", kDuoExtDefault))) {
-    // Default path for all-revolute trees whose stash fits Tensor Memory: see launch_duo
-    constexpr int kTmWarps = sizeof(T) == 4 ? 8 : 4;
-    bool used = false;
-    const int rc = wext ? launch_duo<T>(model, aba_kernel_smem_q<T, 0, true>, aba_kernel_tmem_q<T, 512, 0, kTmWarps, true>,
-                                        kTmWarps, M, a, rows, sr, stream, used)
-                        : launch_duo<T>(model, aba_kernel_smem_q<T, 0, false>, aba_kernel_tmem_q<T, 512, 0, kTmWarps, false>,
-                                        kTmWarps, M, a, rows, 0, stream, used);
-    if (rc) return rc;
-    if (used) return RBD_OK;
-  }
-  if (hm.general) return wext ? RBD_ABA(true, true, kAllKinds) : RBD_ABA(true, false, kAllKinds);
-  if (other_kinds) return wext ? RBD_ABA(false, true, kAllKinds) : RBD_ABA(false, false, kAllKinds);
-  return wext ? RBD_ABA(false, true, 0) : RBD_ABA(false, false, 0);
-#undef RBD_ABA
+    return launch_generic_aba<T>(hm, a, wext != nullptr, stream);
+  };
+  if (wext) return generic(nullptr);      // the model-specialised kernels take no external wrenches
+  SpecKey key; key.algo = SPEC_ABA; key.f64 = sizeof(T) == 8; key.has_in2 = tau != nullptr; key.has_out1 = qd != nullptr;
+  return spec_or_generic(model, key, {q, v, tau, vd, qd, ld, B}, stream, generic);
 }
 
 template <class T>
@@ -656,37 +650,22 @@ int inverse_dynamics_t(const rbd_model* model, int64_t B, int64_t ld, const void
   const ModelDev<T>& M = dev_model<T>(hm);
   RneaArgs<T> a{(const T*)q, (const T*)v, (const T*)vd, (const T*)wext, (T*)tau, nullptr, ld, B};
   const int rows = rnea_rows(hm);
-  if (!wext) {
-    SpecKey key; key.algo = SPEC_RNEA; key.f64 = sizeof(T) == 8; key.has_in2 = vd != nullptr;
-    const SpecLaunchArgs sa{q, v, vd, tau, nullptr, ld, B};
-    bool used = false;
-    std::string err;
-    const int* gate = nullptr;
-    if (int rc = spec_try_launch(const_cast<rbd_model*>(model), key, sa, stream, used, g_launch, &gate, err)) return fail(rc, err);
-    if (used) {
-      g_launch.specialised = 1;
-      if (!gate) return RBD_OK;
-      const rbd_launch_info keep = g_launch;      // gated generic fallback, see dynamics_t
-      a.gate = gate;
-      const int rc = launch<T>(rnea_kernel<T, kNT, false>, M, a, kNT, rows, 0, stream);
-      const int n = g_launch.kernels_launched;
-      g_launch = keep;
-      g_launch.kernels_launched = n;
-      return rc;
+  const int sr = wext ? 6 * hm.nb : 0;
+  auto generic = [&](const int* gate) {
+    a.gate = gate;
+    if (!gate && rows <= 256) {      // the kernel pair, see dynamics_t
+      constexpr int kTmWarps = sizeof(T) == 4 ? 8 : 4;
+      bool used = false;
+      const int rc = launch_duo<T>(model, wext ? rnea_kernel_smem_q<T, true> : rnea_kernel_smem_q<T, false>,
+                                   wext ? rnea_kernel_tmem_q<T, 512, kTmWarps, true> : rnea_kernel_tmem_q<T, 512, kTmWarps, false>,
+                                   kTmWarps, M, a, rows, sr, stream, used);
+      if (rc || used) return rc;
     }
-  }
-  if (rows <= 256 && duo_enabled("RBD_DUO_RNEA", kDuoRneaDefault) && (!wext || duo_enabled("RBD_DUO_EXT", kDuoExtDefault))) {
-    constexpr int kTmWarps = sizeof(T) == 4 ? 8 : 4;
-    bool used = false;
-    const int rc = wext ? launch_duo<T>(model, rnea_kernel_smem_q<T, true>, rnea_kernel_tmem_q<T, 512, kTmWarps, true>, kTmWarps,
-                                        M, a, rows, 6 * hm.nb, stream, used)
-                        : launch_duo<T>(model, rnea_kernel_smem_q<T, false>, rnea_kernel_tmem_q<T, 512, kTmWarps, false>, kTmWarps,
-                                        M, a, rows, 0, stream, used);
-    if (rc) return rc;
-    if (used) return RBD_OK;
-  }
-  return wext ? launch<T>(rnea_kernel<T, kNT, true>, M, a, kNT, rows, 6 * hm.nb, stream)
-              : launch<T>(rnea_kernel<T, kNT, false>, M, a, kNT, rows, 0, stream);
+    return launch<T>(wext ? rnea_kernel<T, kNT, true> : rnea_kernel<T, kNT, false>, kNT, rows, B, &a.scratch, sr, stream, M, a);
+  };
+  if (wext) return generic(nullptr);
+  SpecKey key; key.algo = SPEC_RNEA; key.f64 = sizeof(T) == 8; key.has_in2 = vd != nullptr;
+  return spec_or_generic(model, key, {q, v, vd, tau, nullptr, ld, B}, stream, generic);
 }
 
 template <class T>
@@ -697,28 +676,13 @@ int mass_matrix_t(const rbd_model* model, int64_t B, int64_t ld, const void* q, 
   const int rows = std::max(1, crba_rows(hm));
   bool multi = false;
   for (int i = 0; i < hm.nb; ++i) multi |= kind_nv(M.body[i].kind) > 1;
-  {      // model-specialised kernel: the composite-rigid-body algorithm traced on this mechanism (rbd_codegen.cpp)
-    SpecKey key; key.algo = SPEC_CRBA; key.f64 = sizeof(T) == 8; key.has_in2 = false; key.lower = lower;
-    const SpecLaunchArgs sa{q, nullptr, nullptr, Mout, nullptr, ld, B};
-    bool used = false;
-    std::string err;
-    const int* gate = nullptr;
-    if (int rc = spec_try_launch(const_cast<rbd_model*>(model), key, sa, stream, used, g_launch, &gate, err)) return fail(rc, err);
-    if (used) {
-      g_launch.specialised = 1;
-      if (!gate) return RBD_OK;
-      const rbd_launch_info keep = g_launch;      // gated generic fallback, see dynamics_t
-      a.gate = gate;
-      const int rc = multi ? launch<T>(crba_kernel<T, kNT, 6>, M, a, kNT, rows, 0, stream)
-                           : launch<T>(crba_kernel<T, kNT, 1>, M, a, kNT, rows, 0, stream);
-      const int n = g_launch.kernels_launched;
-      g_launch = keep;
-      g_launch.kernels_launched = n;
-      return rc;
-    }
-  }
-  return multi ? launch<T>(crba_kernel<T, kNT, 6>, M, a, kNT, rows, 0, stream)
-               : launch<T>(crba_kernel<T, kNT, 1>, M, a, kNT, rows, 0, stream);
+  auto generic = [&](const int* gate) {
+    a.gate = gate;
+    return launch<T>(multi ? crba_kernel<T, kNT, 6> : crba_kernel<T, kNT, 1>, kNT, rows, B, nullptr, 0, stream, M, a);
+  };
+  // model-specialised kernel: the composite-rigid-body algorithm traced on this mechanism (rbd_codegen.cpp)
+  SpecKey key; key.algo = SPEC_CRBA; key.f64 = sizeof(T) == 8; key.has_in2 = false; key.lower = lower;
+  return spec_or_generic(model, key, {q, nullptr, nullptr, Mout, nullptr, ld, B}, stream, generic);
 }
 
 // Kinematics by-products (SURVEY 8(f) rank 2).  One launch; the momentum matrix additionally parks the 12 nb pose rows of
@@ -738,45 +702,20 @@ int kinematics_t(const rbd_model* model, int64_t B, int64_t ld, const void* q, c
   KinArgs<T> a{(const T*)q, (const T*)v, (T*)o.transforms_to_root, (T*)o.center_of_mass, (T*)o.kinetic_energy,
                (T*)o.gravitational_potential_energy, (T*)o.momentum, (T*)o.momentum_rate_bias, (T*)o.momentum_matrix,
                (T*)o.geometric_jacobian, nullptr, ld, B, nullptr};
-  DeviceProps p;
-  if (int rc = get_props(p)) return rc;
-  {                              // model-specialised kernel for this output subset (and this jacobian path)
-    SpecKey key;
-    key.algo = SPEC_KIN; key.f64 = sizeof(T) == 8; key.has_in2 = v != nullptr;
-    void* const outs[8] = {o.transforms_to_root, o.center_of_mass, o.kinetic_energy, o.gravitational_potential_energy, o.momentum,
-                           o.momentum_rate_bias, o.momentum_matrix, o.geometric_jacobian};
-    SpecLaunchArgs sa{q, v, nullptr, nullptr, nullptr, ld, B};
-    for (int k = 0; k < 8; ++k) { if (outs[k]) key.kin_mask |= 1 << k; sa.ko[k] = outs[k]; }
-    for (int i = 0; i < hm.nb; ++i) key.kin_sign[i] = K.sign[i];
-    bool used = false;
-    std::string err;
-    const int* gate = nullptr;
-    if (key.kin_mask)
-      if (int rc = spec_try_launch(const_cast<rbd_model*>(model), key, sa, stream, used, g_launch, &gate, err)) return fail(rc, err);
-    if (used) {
-      g_launch.specialised = 1;
-      if (!gate) return RBD_OK;
-      a.gate = gate;               // gated generic fallback (angles beyond the fast sin / cos range), see dynamics_t
-    }
-  }
-  auto kernel = kin_kernel<T, kNT>;
-  const size_t smem = (size_t)std::max(1, kin_rows(hm)) * kNT * sizeof(T);
-  int bps = 0;
-  if (int rc = configure(kernel, kNT, smem, p, bps)) return rc;
-  const int64_t ngroups = (B + kNT - 1) / kNT;
-  const int grid = (int)std::min<int64_t>(ngroups, (int64_t)bps * p.sms);
-  void* scratch = nullptr;
-  if (o.momentum_matrix) {
-    CUDA_TRY(cudaMallocAsync(&scratch, (size_t)12 * hm.nb * grid * kNT * sizeof(T), stream));
-    a.scratch = (T*)scratch;
-  }
-  kernel<<<grid, kNT, smem, stream>>>(M, a, K);
-  cudaError_t e = cudaGetLastError();
-  if (scratch) cudaFreeAsync(scratch, stream);
-  if (e != cudaSuccess) return fail_cuda(e, "kernel launch");
-  g_launch.kernels_launched += 1;
-  g_launch.grid = grid; g_launch.block = kNT; g_launch.smem_bytes = (int)smem; g_launch.blocks_per_sm = bps;
-  return RBD_OK;
+  auto generic = [&](const int* gate) {
+    a.gate = gate;
+    return launch<T>(kin_kernel<T, kNT>, kNT, std::max(1, kin_rows(hm)), B, &a.scratch, o.momentum_matrix ? 12 * hm.nb : 0, stream,
+                     M, a, K);
+  };
+  // model-specialised kernel for this output subset (and this jacobian path)
+  SpecKey key;
+  key.algo = SPEC_KIN; key.f64 = sizeof(T) == 8; key.has_in2 = v != nullptr;
+  void* const outs[8] = {o.transforms_to_root, o.center_of_mass, o.kinetic_energy, o.gravitational_potential_energy, o.momentum,
+                         o.momentum_rate_bias, o.momentum_matrix, o.geometric_jacobian};
+  SpecLaunchArgs sa{q, v, nullptr, nullptr, nullptr, ld, B};
+  for (int k = 0; k < 8; ++k) { if (outs[k]) key.kin_mask |= 1 << k; sa.ko[k] = outs[k]; }
+  for (int i = 0; i < hm.nb; ++i) key.kin_sign[i] = K.sign[i];
+  return key.kin_mask ? spec_or_generic(model, key, sa, stream, generic) : generic(nullptr);
 }
 
 // dynamics! on Dual{Float64,6} arrays (config 4).  The Dual model (constants with zero partials, 25 KB) is built per call
@@ -802,9 +741,9 @@ int dynamics_dual(const rbd_model* model, int64_t B, int64_t ld, const void* q, 
   const DualArgs a{(const double*)q, (const double*)v, (const double*)tau, (double*)vd, ld, B};
   DeviceProps p;
   if (int rc = get_props(p)) return rc;
-  // split stash (shared memory + Tensor Memory): 4 warps/SM instead of 2 on Atlas
+  // split stash (shared memory + Tensor Memory): 4 warps/SM instead of 2 on Atlas; one CTA per SM, it takes all 512 columns
   const size_t smem_tm = (size_t)S.nrows * 128 * sizeof(double);
-  if (!hm.general && S.nrows <= 256 && (int)smem_tm <= p.max_smem_optin && B * 6 >= (int64_t)p.sms * 128 && !getenv("RBD_NO_TMEM")) {
+  if (!hm.general && S.nrows <= 256 && (int)smem_tm <= p.max_smem_optin && B * 6 >= (int64_t)p.sms * 128 && !launch_env().no_tmem) {
     int bps_tm = 0;
     if (int rc = configure(aba_dual_kernel_tm, 128, smem_tm, p, bps_tm)) return rc;
     const int64_t ng = (B * 6 + 127) / 128;
@@ -815,18 +754,9 @@ int dynamics_dual(const rbd_model* model, int64_t B, int64_t ld, const void* q, 
     g_launch.grid = grid_tm; g_launch.block = 128; g_launch.smem_bytes = (int)smem_tm; g_launch.blocks_per_sm = 1;
     return RBD_OK;
   }
-  const size_t smem = (size_t)S.nrows * kNT * sizeof(Dual64);
-  int bps = 0;
-  if (int rc = hm.general ? configure(aba_dual_kernel<kNT, true>, kNT, smem, p, bps)
-                          : configure(aba_dual_kernel<kNT, false>, kNT, smem, p, bps)) return rc;
-  const int64_t ngroups = (B * 6 + kNT - 1) / kNT;      // one thread per (sample, partial direction)
-  const int grid = (int)std::min<int64_t>(ngroups, (int64_t)bps * p.sms);
-  if (hm.general) aba_dual_kernel<kNT, true><<<grid, kNT, smem, stream>>>(*Mp, a);
-  else aba_dual_kernel<kNT, false><<<grid, kNT, smem, stream>>>(*Mp, a);
-  CUDA_TRY(cudaGetLastError());
-  g_launch.kernels_launched += 1;
-  g_launch.grid = grid; g_launch.block = kNT; g_launch.smem_bytes = (int)smem; g_launch.blocks_per_sm = bps;
-  return RBD_OK;
+  // one thread per (sample, partial direction)
+  return launch<Dual64>(hm.general ? aba_dual_kernel<kNT, true> : aba_dual_kernel<kNT, false>, kNT, S.nrows, B * 6, nullptr, 0, stream,
+                        *Mp, a);
 }
 
 // ---- Munthe-Kaas RK4 (rbd_integrate): elementwise stage kernels around the dynamics kernels -----------------------------
@@ -1093,94 +1023,55 @@ template <class T>
 int dynamics_gather_t(const rbd_model* model, int64_t B, int64_t ld, const void* q, const void* v, const void* tau, int npeers,
                       void* const* peers, void* mc, int64_t peer_ld, int64_t col0, cudaStream_t stream) {
   const HostModel& hm = model->hm;
-  const ModelDev<T>& M = dev_model<T>(hm);
-  const int* gate = nullptr;
-  bool used = false;
-  {
-    SpecKey key; key.algo = SPEC_ABA; key.f64 = sizeof(T) == 8; key.has_in2 = tau != nullptr; key.peers = true;
-    SpecLaunchArgs sa{q, v, tau, nullptr, nullptr, ld, B};
-    sa.peers = peers; sa.npeers = npeers; sa.peer_ld = peer_ld; sa.peer_col0 = col0; sa.mc = mc;
-    std::string err;
-    if (int rc = spec_try_launch(const_cast<rbd_model*>(model), key, sa, stream, used, g_launch, &gate, err)) return fail(rc, err);
-    if (used) g_launch.specialised = 1;
-    if (used && !gate) return RBD_OK;
-  }
-  const rbd_launch_info keep = g_launch;
-  // the generic kernels use ONE leading dimension for inputs and outputs, so the scratch is [nv x ld]
-  T* scratch = nullptr;
-  CUDA_TRY(cudaMallocAsync((void**)&scratch, (size_t)hm.nv * (size_t)ld * sizeof(T), stream));
-  int rc;
-  if (!used) {
-    rc = dynamics_t<T>(model, B, ld, q, v, tau, nullptr, scratch, nullptr, stream);
-  } else {
-    AbaArgs<T> a{(const T*)q, (const T*)v, (const T*)tau, nullptr, scratch, nullptr, nullptr, ld, B};
-    a.gate = gate;
-    bool other_kinds = false;
-    for (int i = 0; i < hm.nb; ++i) other_kinds |= (M.body[i].kind == K_PRIS || M.body[i].kind == K_FIXED);
-    const int rows = M.nrows;
-#define RBD_ABA_G(G, K) launch<T>(aba_kernel<T, kNT, G, false, K>, M, a, kNT, rows, 0, stream)
-    rc = hm.general ? RBD_ABA_G(true, kAllKinds) : (other_kinds ? RBD_ABA_G(false, kAllKinds) : RBD_ABA_G(false, 0));
-#undef RBD_ABA_G
-  }
-  if (rc == RBD_OK) {
-    ScatterArgs<T> sc{};
-    sc.src = scratch; sc.src_ld = ld; sc.dst_ld = peer_ld; sc.ndst = npeers; sc.rows = hm.nv; sc.B = B; sc.gate = gate;
-    for (int p = 0; p < npeers; ++p) sc.dst[p] = (T*)peers[p] + col0;
-    DeviceProps p;
-    if ((rc = get_props(p)) == RBD_OK) {
-      gather_scatter_kernel<T><<<p.sms * 8, 256, 0, stream>>>(sc);
-      if (cudaGetLastError() != cudaSuccess) rc = fail(RBD_ECUDA, "gather_scatter_kernel launch failed");
-      g_launch.kernels_launched += 1;
+  // generic kernels: they use ONE leading dimension for inputs and outputs, so they write into a [nv x ld] scratch which
+  // gather_scatter_kernel then copies to the peers
+  auto generic = [&](const int* gate) {
+    T* scratch = nullptr;
+    CUDA_TRY(cudaMallocAsync((void**)&scratch, (size_t)hm.nv * (size_t)ld * sizeof(T), stream));
+    int rc;
+    if (gate) {        // behind the peer-writing specialised kernel
+      AbaArgs<T> a{(const T*)q, (const T*)v, (const T*)tau, nullptr, scratch, nullptr, nullptr, ld, B};
+      a.gate = gate;
+      rc = launch_generic_aba<T>(hm, a, false, stream);
+    } else {
+      rc = dynamics_t<T>(model, B, ld, q, v, tau, nullptr, scratch, nullptr, stream);
     }
-  }
-  cudaFreeAsync(scratch, stream);
-  const int n = g_launch.kernels_launched;
-  if (used) { g_launch = keep; g_launch.kernels_launched = n; }
-  return rc;
+    if (rc == RBD_OK) {
+      ScatterArgs<T> sc{};
+      sc.src = scratch; sc.src_ld = ld; sc.dst_ld = peer_ld; sc.ndst = npeers; sc.rows = hm.nv; sc.B = B; sc.gate = gate;
+      for (int p = 0; p < npeers; ++p) sc.dst[p] = (T*)peers[p] + col0;
+      DeviceProps p;
+      if ((rc = get_props(p)) == RBD_OK) {
+        gather_scatter_kernel<T><<<p.sms * 8, 256, 0, stream>>>(sc);
+        if (cudaGetLastError() != cudaSuccess) rc = fail(RBD_ECUDA, "gather_scatter_kernel launch failed");
+        g_launch.kernels_launched += 1;
+      }
+    }
+    cudaFreeAsync(scratch, stream);
+    return rc;
+  };
+  SpecKey key; key.algo = SPEC_ABA; key.f64 = sizeof(T) == 8; key.has_in2 = tau != nullptr; key.peers = true;
+  SpecLaunchArgs sa{q, v, tau, nullptr, nullptr, ld, B};
+  sa.peers = peers; sa.npeers = npeers; sa.peer_ld = peer_ld; sa.peer_col0 = col0; sa.mc = mc;
+  return spec_or_generic(model, key, sa, stream, generic);
 }
 
 template <class T>
 int bodies_t(const rbd_model* model, int64_t B, int64_t ld, const void* q, const void* v, const void* vd, const void* wext, void* acc,
              void* jw, cudaStream_t stream) {
   const HostModel& hm = model->hm;
-  const ModelDev<T>& M = dev_model<T>(hm);
-  BodiesArgs<T> a{(const T*)q, (const T*)v, (const T*)vd, (const T*)wext, (T*)acc, (T*)jw, ld, B};
-  DeviceProps p;
-  if (int rc = get_props(p)) return rc;
-  auto kernel = bodies_kernel<T, kNT>;
-  const size_t smem = (size_t)std::max(1, kin_rows(hm)) * kNT * sizeof(T);
-  int bps = 0;
-  if (int rc = configure(kernel, kNT, smem, p, bps)) return rc;
-  const int64_t ngroups = (B + kNT - 1) / kNT;
-  const int grid = (int)std::min<int64_t>(ngroups, (int64_t)bps * p.sms);
-  kernel<<<grid, kNT, smem, stream>>>(M, a);
-  if (cudaGetLastError() != cudaSuccess) return fail(RBD_ECUDA, "bodies_kernel launch failed");
-  g_launch.kernels_launched += 1;
-  g_launch.grid = grid; g_launch.block = kNT; g_launch.smem_bytes = (int)smem; g_launch.blocks_per_sm = bps;
-  return RBD_OK;
+  const BodiesArgs<T> a{(const T*)q, (const T*)v, (const T*)vd, (const T*)wext, (T*)acc, (T*)jw, ld, B};
+  return launch<T>(bodies_kernel<T, kNT>, kNT, std::max(1, kin_rows(hm)), B, nullptr, 0, stream, dev_model<T>(hm), a);
 }
 
 template <class T>
 int contact_t(const rbd_model* model, int64_t B, int64_t ld, const void* q, const void* v, const rbd_contact_desc& cd, void* sx,
               void* sd, void* wr, cudaStream_t stream) {
   const HostModel& hm = model->hm;
-  const ModelDev<T>& M = dev_model<T>(hm);
   ContactDev<T> C;
   build_contact_dev<T>(hm.nb, hm.pos.data(), hm.alignT.data(), cd, C);
-  ContactArgs<T> a{(const T*)q, (const T*)v, (T*)sx, (T*)sd, (T*)wr, ld, B};
-  DeviceProps p;
-  if (int rc = get_props(p)) return rc;
-  auto kernel = contact_kernel<T, kNT>;
-  const size_t smem = (size_t)std::max(1, kin_rows(hm)) * kNT * sizeof(T);
-  int bps = 0;
-  if (int rc = configure(kernel, kNT, smem, p, bps)) return rc;
-  const int64_t ngroups = (B + kNT - 1) / kNT;
-  const int grid = (int)std::min<int64_t>(ngroups, (int64_t)bps * p.sms);
-  kernel<<<grid, kNT, smem, stream>>>(M, C, a);
-  if (cudaGetLastError() != cudaSuccess) return fail(RBD_ECUDA, "contact_kernel launch failed");
-  g_launch.kernels_launched += 1;
-  g_launch.grid = grid; g_launch.block = kNT; g_launch.smem_bytes = (int)smem; g_launch.blocks_per_sm = bps;
-  return RBD_OK;
+  const ContactArgs<T> a{(const T*)q, (const T*)v, (T*)sx, (T*)sd, (T*)wr, ld, B};
+  return launch<T>(contact_kernel<T, kNT>, kNT, std::max(1, kin_rows(hm)), B, nullptr, 0, stream, dev_model<T>(hm), C, a);
 }
 
 int check_common(const rbd_model* model, int32_t dtype, int64_t B, int64_t ld, bool allow_dual = false) {
@@ -1247,15 +1138,6 @@ int ensure_staging(rbd_model* m, size_t bytes_per_stream) {
   return RBD_OK;
 }
 
-// copy rows x C block between a host array with leading dimension ld and a dense device tile (leading dimension C)
-int copy_rows(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, int rows, cudaMemcpyKind kind,
-              cudaStream_t s) {
-  CUDA_TRY(cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, kind, s));
-  return RBD_OK;
-}
-}  // namespace
-
-namespace {
 struct HostArr { const void* in; void* out; int rows; };
 
 // Chunked host pipeline: chunk c uses stream c % 3 and that stream's staging buffer; H2D copies, the kernel and the D2H
@@ -1296,7 +1178,7 @@ int host_pipeline_impl(rbd_model* model, int32_t dtype, int64_t B, int64_t ld, c
     for (int i = 0; i < nin; ++i) {
       if (!ins[i].in) continue;
       din[i] = cur;
-      if (int rc = copy_rows(cur, C * es, (const char*)ins[i].in + off, ld * es, n * es, ins[i].rows, cudaMemcpyHostToDevice, s)) return rc;
+      CUDA_TRY(cudaMemcpy2DAsync(cur, C * es, (const char*)ins[i].in + off, ld * es, n * es, ins[i].rows, cudaMemcpyHostToDevice, s));
       cur += (size_t)ins[i].rows * C * es;
     }
     for (int i = 0; i < nout; ++i) {
@@ -1304,12 +1186,13 @@ int host_pipeline_impl(rbd_model* model, int32_t dtype, int64_t B, int64_t ld, c
       dout[i] = cur;
       cur += (size_t)outs[i].rows * C * es;
     }
+    g_launch.kernels_launched = 0;
     if (int rc = launch_chunk(n, C, din, dout, s)) return rc;
     launches += g_launch.kernels_launched;
     last = g_launch;
     for (int i = 0; i < nout; ++i) {
       if (!outs[i].out) continue;
-      if (int rc = copy_rows((char*)outs[i].out + off, ld * es, dout[i], C * es, n * es, outs[i].rows, cudaMemcpyDeviceToHost, s)) return rc;
+      CUDA_TRY(cudaMemcpy2DAsync((char*)outs[i].out + off, ld * es, dout[i], C * es, n * es, outs[i].rows, cudaMemcpyDeviceToHost, s));
     }
   }
   for (int i = 0; i < 3; ++i) CUDA_TRY(cudaStreamSynchronize(model->streams[i]));
@@ -1573,9 +1456,6 @@ int32_t rbd_mass_matrix(const rbd_model* model, int32_t dtype, int64_t B, int64_
   return rbd_mass_matrix_uplo(model, dtype, B, ld, q, M_out, RBD_UPLO_FULL, stream);
 }
 
-// ---- host-pointer variants: chunked H2D -> kernel -> D2H pipeline over three internal streams -----------------------
-
-
 int32_t rbd_dynamics_host(rbd_model* model, int32_t dtype, int64_t B, int64_t ld, const void* q, const void* v,
                           const void* tau, const void* wext, void* vd_out, void* qd_out) {
   if (int rc = check_common(model, dtype, B, ld)) return rc;
@@ -1587,7 +1467,6 @@ int32_t rbd_dynamics_host(rbd_model* model, int32_t dtype, int64_t B, int64_t ld
   const HostArr outs[2] = {{nullptr, vd_out, hm.nv}, {nullptr, qd_out, hm.nq}};
   return host_pipeline(model, dtype, B, ld, ins, 4, outs, 2,
                        [&](int64_t n, int64_t C, const void** di, void** dq, cudaStream_t s) {
-                         g_launch.kernels_launched = 0;
                          return dtype == RBD_F32 ? dynamics_t<float>(model, n, C, di[0], di[1], di[2], di[3], dq[0], dq[1], s)
                                                  : dynamics_t<double>(model, n, C, di[0], di[1], di[2], di[3], dq[0], dq[1], s);
                        });
@@ -1604,7 +1483,6 @@ int32_t rbd_inverse_dynamics_host(rbd_model* model, int32_t dtype, int64_t B, in
   const HostArr outs[1] = {{nullptr, tau_out, hm.nv}};
   return host_pipeline(model, dtype, B, ld, ins, 4, outs, 1,
                        [&](int64_t n, int64_t C, const void** di, void** dq, cudaStream_t s) {
-                         g_launch.kernels_launched = 0;
                          return dtype == RBD_F32 ? inverse_dynamics_t<float>(model, n, C, di[0], di[1], di[2], di[3], dq[0], s)
                                                  : inverse_dynamics_t<double>(model, n, C, di[0], di[1], di[2], di[3], dq[0], s);
                        });
@@ -1621,7 +1499,6 @@ int32_t rbd_dynamics_bias_host(rbd_model* model, int32_t dtype, int64_t B, int64
   const HostArr outs[1] = {{nullptr, c_out, hm.nv}};
   return host_pipeline(model, dtype, B, ld, ins, 3, outs, 1,
                        [&](int64_t n, int64_t C, const void** di, void** dq, cudaStream_t s) {
-                         g_launch.kernels_launched = 0;
                          return dtype == RBD_F32 ? inverse_dynamics_t<float>(model, n, C, di[0], di[1], nullptr, di[2], dq[0], s)
                                                  : inverse_dynamics_t<double>(model, n, C, di[0], di[1], nullptr, di[2], dq[0], s);
                        });
@@ -1637,7 +1514,6 @@ int32_t rbd_mass_matrix_host(rbd_model* model, int32_t dtype, int64_t B, int64_t
   const HostArr outs[1] = {{nullptr, M_out, hm.nv * hm.nv}};
   return host_pipeline(model, dtype, B, ld, ins, 1, outs, 1,
                        [&](int64_t n, int64_t C, const void** di, void** dq, cudaStream_t s) {
-                         g_launch.kernels_launched = 0;
                          return dtype == RBD_F32 ? mass_matrix_t<float>(model, n, C, di[0], dq[0], s)
                                                  : mass_matrix_t<double>(model, n, C, di[0], dq[0], s);
                        });

@@ -20,7 +20,6 @@
 #include <cstring>
 #include <map>
 #include <mutex>
-#include <set>
 #include <string>
 #include <vector>
 
@@ -148,28 +147,6 @@ __global__ void deriv_solve_kernel(const __grid_constant__ DerivDev D, const __g
   }
 }
 
-struct Props { int dev = 0, sms = 0, max_smem_optin = 0, smem_per_sm = 0; };
-int get_props(Props& p) {
-  if (cudaGetDevice(&p.dev) != cudaSuccess) return api_fail(RBD_ECUDA, "cudaGetDevice failed");
-  cudaDeviceGetAttribute(&p.sms, cudaDevAttrMultiProcessorCount, p.dev);
-  cudaDeviceGetAttribute(&p.max_smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, p.dev);
-  cudaDeviceGetAttribute(&p.smem_per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, p.dev);
-  return RBD_OK;
-}
-// opt a kernel into large dynamic shared memory once per (kernel, device)
-int big_smem_once(const void* kernel, const Props& p) {
-  static std::mutex mu;
-  static std::set<std::pair<const void*, int>> done;
-  std::lock_guard<std::mutex> lk(mu);
-  if (done.count({kernel, p.dev})) return RBD_OK;
-  cudaFuncAttributes fa{};
-  if (cudaFuncGetAttributes(&fa, kernel) != cudaSuccess ||
-      cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, p.max_smem_optin - (int)fa.sharedSizeBytes) != cudaSuccess)
-    return api_fail(RBD_ECUDA, std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(cudaGetLastError()));
-  cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  done.insert({kernel, p.dev});
-  return RBD_OK;
-}
 #define LAUNCH_CHECK(name) do { cudaError_t e_ = cudaGetLastError(); if (e_ != cudaSuccess) { rc = api_fail(RBD_ECUDA, std::string(name " launch failed: ") + cudaGetErrorString(e_)); goto done; } } while (0)
 
 // ---- model-specialised solve kernel (rbd_deriv_jit.cpp): compiled with NVRTC on the first large call (or ahead of time by
@@ -208,7 +185,7 @@ bool jit_solve_cubin(const DerivDev& D, const DerivAnc& A, bool f64, bool compil
   bool from_cache = false;
   return jit_compile_text(f64 ? "deriv_f64" : "deriv_f32", src, true, cubin, compile, &from_cache, err);
 }
-JitSolve* jit_solve_get(const DerivDev& D, const DerivAnc& A, bool f64, int64_t B, const Props& p) {
+JitSolve* jit_solve_get(const DerivDev& D, const DerivAnc& A, bool f64, int64_t B, const DeviceProps& p) {
   if (!jit_enabled()) return nullptr;
   std::string key((const char*)&D, sizeof(D));
   key.append((const char*)A.anc, sizeof(int16_t) * D.nnz);
@@ -254,7 +231,7 @@ int derivatives_t(const rbd_model* model, int32_t dtype, int64_t B, int64_t ld, 
   if (!build_deriv_dev(M, D, A))
     return api_fail(RBD_EUNSUPPORTED, "rbd_dynamics_derivatives: more than 128 velocity coordinates or 4096 mass-matrix entries");
   if (D.nv == 0) return RBD_OK;        // nothing to differentiate (only fixed joints): no outputs have any rows
-  Props p;
+  DeviceProps p;
   if (int rc = get_props(p)) return rc;
   // chunk size from the scratch budget
   int64_t budget_mb = 2048;
@@ -290,8 +267,8 @@ int derivatives_t(const rbd_model* model, int32_t dtype, int64_t B, int64_t ld, 
   auto kworld = deriv_world_kernel<T, kNT>;
   auto ksolve_s = deriv_solve_kernel<T, true>;
   auto ksolve_g = deriv_solve_kernel<T, false>;
-  if ((rc = big_smem_once((const void*)kworld, p)) != RBD_OK) goto done;
-  if ((rc = big_smem_once(hs ? (const void*)ksolve_s : (const void*)ksolve_g, p)) != RBD_OK) goto done;
+  if ((rc = configure_once((const void*)kworld, p)) != RBD_OK) goto done;
+  if ((rc = configure_once(hs ? (const void*)ksolve_s : (const void*)ksolve_g, p)) != RBD_OK) goto done;
   if (world_smem > (size_t)p.max_smem_optin) { rc = api_fail(RBD_EUNSUPPORTED, "rbd_dynamics_derivatives: too many open branch nodes"); goto done; }
   for (int64_t b0 = 0; b0 < B; b0 += C) {
     const int64_t c = std::min<int64_t>(C, B - b0);

@@ -1,8 +1,9 @@
-// The opaque model handle of the C ABI (include/rbd_b200.h), shared by rbd_b200.cu (generic kernels, entry points) and
-// rbd_spec.cpp (model-specialised kernels).
+// The opaque model handle of the C ABI (include/rbd_b200.h), shared by rbd_b200.cu (generic kernels, entry points),
+// rbd_spec.cpp (model-specialised kernels) and rbd_deriv.cu (derivatives), with the launch plumbing they have in common.
 #pragma once
 #include <cuda_runtime.h>
 
+#include <cstdlib>
 #include <map>
 #include <mutex>
 #include <string>
@@ -89,12 +90,45 @@ struct SpecLaunchArgs {
 // Tries the model-specialised kernels for (model, key).  `used` = false (and RBD_OK) when they are unavailable, not yet
 // compiled and the batch is below the compile threshold, or the batch is too small: the caller then runs the generic kernels.
 // `gate` (fp32 only, else NULL): device flag the specialised kernels raise when a sample needs the library sin / cos; the caller
-// must enqueue the generic kernel gated on it right behind.
+// must enqueue the generic kernel gated on it right behind.  Errors are reported through api_fail.
 int spec_try_launch(rbd_model* m, const SpecKey& key, const SpecLaunchArgs& a, cudaStream_t stream, bool& used,
-                    rbd_launch_info& li, const int** gate, std::string& err);
+                    rbd_launch_info& li, const int** gate);
 // Compile (or load from the cubin cache) without launching; RBD_OK / RBD_EUNSUPPORTED.
 int spec_prepare(rbd_model* m, const SpecKey& key, bool load_on_device, std::string& err);
 void spec_release(rbd_model* m);
+
+// Launch switches (DESIGN.md §4.7), read once per process.
+struct LaunchEnv {
+  bool jit = true;                  // RBD_JIT=0: generic kernels only
+  int64_t jit_min_batch = 1 << 15;  // below this a missing cubin is not compiled on the fly (generic kernels serve the call)
+  int jit_variant = 0;              // RBD_JIT_VARIANT=1 (pair) / 2 (unified): skip the tuning
+  bool jit_verbose = false;         // RBD_JIT_VERBOSE: print why a specialised kernel is unavailable
+  bool no_tmem = false;             // RBD_NO_TMEM: single-kernel paths only
+  bool no_gate = false;             // RBD_NO_GATE: no generic kernel behind the fp32 specialised ones (profile captures)
+  const char* only = nullptr;       // RBD_ONLY=smem|tmem: launch one kernel of a pair (ncu captures: the profiler serialises them)
+  LaunchEnv() {
+    if (const char* e = getenv("RBD_JIT")) jit = e[0] != '0';
+    if (const char* e = getenv("RBD_JIT_MIN_BATCH")) jit_min_batch = atoll(e);
+    if (const char* e = getenv("RBD_JIT_VARIANT")) jit_variant = atoi(e);
+    jit_verbose = getenv("RBD_JIT_VERBOSE") != nullptr;
+    no_tmem = getenv("RBD_NO_TMEM") != nullptr;
+    no_gate = getenv("RBD_NO_GATE") != nullptr;
+    only = getenv("RBD_ONLY");
+  }
+};
+inline const LaunchEnv& launch_env() { static const LaunchEnv e; return e; }
+
+// Properties of the current device, cached per device.  The first query on a device also keeps freed blocks cached in its
+// stream-ordered memory pool (scratch for slots / external wrenches comes from there).
+struct DeviceProps { int dev = 0; int sms = 0; int max_smem_optin = 0; int smem_per_sm = 0; bool ok = false; };
+int get_props(DeviceProps& p);
+// Opt a kernel into large dynamic shared memory ONCE per (kernel, device): the attribute is process-global per kernel, so
+// setting it to each call's exact size would race between host threads using different model handles.
+int configure_once(const void* kernel, const DeviceProps& p);
+// Blocks per SM of a single-warp shared-memory kernel running next to one Tensor-Memory CTA of `tm_warps` warps on every SM,
+// or 0 when that kernel pair should not be used.  `bps`: the shared-memory kernel's blocks per SM on its own; `regs_*`: the
+// two kernels' registers per thread; `ngroups`: groups of 32 samples in the batch.
+int pair_blocks(int sms, int bps, int regs_smem, int regs_tmem, int tm_warps, int64_t ngroups);
 
 // rbd_b200.cu's per-thread error text / argument checks / launch statistics, for the library's other translation units
 int api_fail(int status, const std::string& msg);

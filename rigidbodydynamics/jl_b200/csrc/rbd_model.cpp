@@ -250,7 +250,7 @@ int build_host_model(const rbd_model_desc* desc, HostModel& out, std::string& er
   for (int i = nb - 1; i >= 0; --i) if (desc->parent[i] >= 0) subtree_size[desc->parent[i]] += subtree_size[i];
   std::vector<int> slot_free_at;          // slot -> first preorder position at which it may be re-used
   int nslots = 0, row = 0;
-  bool general = false;
+  bool general = false, other_kinds = false;
   for (int p = 0; p < nb; ++p) {
     const int j = out.order[p];
     BodyDev<double>& b = M.body[p];
@@ -331,6 +331,7 @@ int build_host_model(const rbd_model_desc* desc, HostModel& out, std::string& er
     const int k = kind_nv(b.kind);
     const bool multi = k > 1;
     if (multi && !(p == 0 && par < 0)) general = true;
+    if (b.kind == K_PRIS || b.kind == K_FIXED) other_kinds = true;
     b.row0 = row;
     if (k <= 1) row += (b.kind == K_FIXED) ? 6 : kRowsOneDof;
     else if (p == 0 && par < 0) row += 6;                 // root multi-DoF joint: only its velocity is stashed
@@ -342,6 +343,7 @@ int build_host_model(const rbd_model_desc* desc, HostModel& out, std::string& er
   M.nrows = row + nslots * kSlotRowsAba;
   out.nslots = nslots;
   out.general = general;
+  out.other_kinds = other_kinds;
   fill_dev(out, M, out.dev32);
   return RBD_OK;
 }

@@ -15,6 +15,7 @@ struct HostModel {
   int64_t modcount = 0;
   int nslots = 0;            // pending slots (max nesting of branch nodes)
   bool general = false;      // multi-DoF joint somewhere other than preorder position 0 under the world
+  bool other_kinds = false;  // prismatic or fixed joints: the generic kernels need those code paths (else revolute-only)
   std::vector<int> order;    // preorder position -> reference joint index
   std::vector<int> pos;      // reference joint index -> preorder position
   std::vector<int> qstart, vstart;   // reference order

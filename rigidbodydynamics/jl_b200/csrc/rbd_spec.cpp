@@ -4,50 +4,12 @@
 // stream and one Tensor-Memory CTA per SM on the handle's side stream, both claiming groups of 32 samples from one counter.
 #include <algorithm>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 
 #include "rbd_handle.h"
 #include "rbd_jit.h"
 
 namespace rbd {
-namespace {
-
-struct Env {
-  bool jit = true, no_tmem = false, force_pair = false, no_gate = false;
-  int64_t min_batch = 1 << 15;      // below this a missing cubin is not compiled on the fly (generic kernels serve the call)
-  int smem_blocks = 0;
-  int variant = 0;                  // RBD_JIT_VARIANT=1 (pair) / 2 (unified): skip the tuning
-  const char* only = nullptr;       // RBD_ONLY=smem|tmem: launch one kernel of the pair (ncu captures: the profiler serialises them)
-  Env() {
-    if (const char* e = getenv("RBD_JIT")) jit = e[0] != '0';
-    no_tmem = getenv("RBD_NO_TMEM") != nullptr;
-    force_pair = getenv("RBD_FORCE_PAIR") != nullptr;       // experiments only
-    no_gate = getenv("RBD_NO_GATE") != nullptr;
-    if (const char* e = getenv("RBD_JIT_MIN_BATCH")) min_batch = atoll(e);
-    if (const char* e = getenv("RBD_SMEM_BLOCKS")) smem_blocks = atoi(e);
-    if (const char* e = getenv("RBD_JIT_VARIANT")) variant = atoi(e);
-    only = getenv("RBD_ONLY");
-  }
-};
-const Env& env() { static const Env e; return e; }
-
-struct Props { int sms = 0, max_smem_optin = 0; };
-cudaError_t props(Props& p) {
-  int dev = 0;
-  cudaError_t e = cudaGetDevice(&dev);
-  if (e != cudaSuccess) return e;
-  static std::mutex mu;
-  static Props cache[64];
-  std::lock_guard<std::mutex> lk(mu);
-  if (dev < 64 && cache[dev].sms) { p = cache[dev]; return cudaSuccess; }
-  if ((e = cudaDeviceGetAttribute(&p.sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-  if ((e = cudaDeviceGetAttribute(&p.max_smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
-  if (dev < 64) cache[dev] = p;
-  return cudaSuccess;
-}
-
-}  // namespace
 
 cudaError_t pair_begin(rbd_model* m, cudaStream_t stream, PairCtx& ctx) {
   int dev = 0;
@@ -93,8 +55,8 @@ void spec_release(rbd_model* m) {
 // are therefore always specialised, fp64 programs only below an estimated size.
 bool spec_worthwhile(const HostModel& hm, const SpecKey& key) {
   if (!key.f64) return true;
-  if (key.algo == SPEC_CRBA) return !getenv("RBD_JIT_NO_CRBA64");   // small stash (2 rows per body): fp64 keeps its resident warps
-  if (key.algo == SPEC_KIN) return true;                             // stash = the pending branch nodes only
+  if (key.algo == SPEC_CRBA) return true;   // small stash (2 rows per body): fp64 keeps its resident warps
+  if (key.algo == SPEC_KIN) return true;    // stash = the pending branch nodes only
   const int est = hm.nb * (key.algo == SPEC_ABA ? 410 : 190);
   return est <= 6500;
 }
@@ -140,16 +102,16 @@ int spec_prepare(rbd_model* m, const SpecKey& key, bool load_on_device, std::str
 }
 
 int spec_try_launch(rbd_model* m, const SpecKey& key, const SpecLaunchArgs& a, cudaStream_t stream, bool& used,
-                    rbd_launch_info& li, const int** gate, std::string& err) {
+                    rbd_launch_info& li, const int** gate) {
   used = false;
   if (gate) *gate = nullptr;
-  const Env& ev = env();
+  const LaunchEnv& ev = launch_env();
   if (!ev.jit || !spec_worthwhile(m->hm, key)) return RBD_OK;
   if (a.ld * (key.f64 ? 8 : 4) >= (1ll << 32)) return RBD_OK;   // the generated code forms row offsets as 32 x 32 -> 64-bit products of the byte stride
   const int rows = spec_stash_rows(m->hm, key);
   if (rows > 256) return RBD_OK;                     // one warp's share of Tensor Memory: 256 fp32 rows (128 x 2 columns in fp64)
-  Props p;
-  if (cudaError_t e = props(p)) { err = cudaGetErrorString(e); return RBD_ECUDA; }
+  DeviceProps p;
+  if (int rc = get_props(p)) return rc;
   const size_t es = key.f64 ? 8 : 4;
   const size_t smem = (size_t)std::max(1, rows) * 32 * es;
   if (smem > (size_t)p.max_smem_optin) return RBD_OK;
@@ -165,7 +127,7 @@ int spec_try_launch(rbd_model* m, const SpecKey& key, const SpecLaunchArgs& a, c
   }
   if (se->state == -1) return RBD_OK;
   if (se->state == 0) {
-    if (a.B < ev.min_batch) {          // small call and nothing loaded yet: use a cached cubin if there is one, never compile
+    if (a.B < ev.jit_min_batch) {          // small call and nothing loaded yet: use a cached cubin if there is one, never compile
       std::vector<char> probe;
       std::string e2;
       bool cached = false;
@@ -173,25 +135,21 @@ int spec_try_launch(rbd_model* m, const SpecKey& key, const SpecLaunchArgs& a, c
     }
     std::string e2;
     if (spec_prepare(m, key, true, e2) != RBD_OK) {      // generic kernels take over; the reason is kept in the entry
-      if (getenv("RBD_JIT_VERBOSE")) fprintf(stderr, "[rbd_b200] specialised kernels unavailable: %s\n", e2.c_str());
+      if (ev.jit_verbose) fprintf(stderr, "[rbd_b200] specialised kernels unavailable: %s\n", e2.c_str());
       return RBD_OK;
     }
   }
   const int64_t ngroups = (a.B + 31) / 32;
   const int tm_warps = key.f64 ? 4 : 8;
   int bps = 0;
-  if (cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, (const void*)se->k_smem, 32, smem)) {
-    err = cudaGetErrorString(e); return RBD_ECUDA;
-  }
+  if (cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, (const void*)se->k_smem, 32, smem))
+    return api_fail(RBD_ECUDA, cudaGetErrorString(e));
   if (bps < 1) return RBD_OK;
   // Three ways to fill an SM (rbd_jit_kernels.cuh): shared-memory blocks alone, the kernel pair, the unified CTA.  The two
   // Tensor-Memory variants are used when they put at least 15 % more warps on the SM than shared memory alone and there is work
   // for them; which of the two is decided by timing both once, on the first call large enough to tell (not while capturing).
-  if (ev.smem_blocks > 0) bps = std::max(1, std::min(bps, ev.smem_blocks));
-  const int rs = ((se->regs_smem + 7) / 8) * 8 * 32, rt = ((se->regs_tmem + 7) / 8) * 8 * 32 * tm_warps;
-  const int bps_pair = std::max(1, std::min(bps, (65536 - rt) / rs));
-  const bool pair_ok = !ev.no_tmem && rt + rs <= 65536 && (bps_pair + tm_warps) * 100 >= bps * 115 &&
-                       ngroups >= (int64_t)(bps_pair + tm_warps / 2) * p.sms;
+  const int bps_pair = ev.no_tmem ? 0 : pair_blocks(p.sms, bps, se->regs_smem, se->regs_tmem, tm_warps, ngroups);
+  const bool pair_ok = bps_pair > 0;
   const int uni_warps = se->uni_sw > 0 ? se->uni_sw + tm_warps : 0;
   const bool uni_ok = !ev.no_tmem && uni_warps * 100 >= bps * 115 && ((se->regs_uni + 7) / 8) * 8 * 32 * uni_warps <= 65536 &&
                       ngroups >= (int64_t)(uni_warps - tm_warps / 2) * p.sms;
@@ -235,7 +193,7 @@ int spec_try_launch(rbd_model* m, const SpecKey& key, const SpecLaunchArgs& a, c
   cudaError_t e = cudaSuccess;
   int variant = 0;
   if (pair_ok && uni_ok) {
-    variant = ev.variant ? ev.variant : se->choice;
+    variant = ev.jit_variant ? ev.jit_variant : se->choice;
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     cudaStreamIsCapturing(stream, &cap);
     if (variant == 0 && cap == cudaStreamCaptureStatusNone && a.B >= (int64_t)p.sms * 32 * 64) {
@@ -260,9 +218,8 @@ int spec_try_launch(rbd_model* m, const SpecKey& key, const SpecLaunchArgs& a, c
     if (variant == 0) variant = 1;
   } else if (uni_ok) variant = 2;
   else if (pair_ok) variant = 1;
-  if (ev.force_pair && uni_warps) variant = 2;
   if (e == cudaSuccess) e = run(variant);
-  if (e != cudaSuccess) { err = std::string("specialised kernel launch: ") + cudaGetErrorString(e); return RBD_ECUDA; }
+  if (e != cudaSuccess) return api_fail(RBD_ECUDA, std::string("specialised kernel launch: ") + cudaGetErrorString(e));
   li.kernels_launched += launched;
   if (gate && !key.f64 && !ev.no_gate) *gate = last_flag;
   used = true;
