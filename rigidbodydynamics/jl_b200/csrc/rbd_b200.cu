@@ -107,10 +107,6 @@ int pair_blocks(int sms, int bps, int regs_smem, int regs_tmem, int tm_warps, in
 
 namespace {
 
-template <class T> const ModelDev<T>& dev_model(const HostModel& m);
-template <> const ModelDev<float>& dev_model<float>(const HostModel& m) { return m.dev32; }
-template <> const ModelDev<double>& dev_model<double>(const HostModel& m) { return m.dev64; }
-
 // ------------------------------------------------------------------------------------------------------------------
 // kernels
 // ------------------------------------------------------------------------------------------------------------------

@@ -18,7 +18,6 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <map>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -30,17 +29,13 @@
 #include "rbd_deriv.cuh"
 #include "rbd_deriv_jit.h"
 #include "rbd_handle.h"
-#include "rbd_jit_text.h"
+#include "rbd_jit.h"
 
 using namespace rbd;
 
 namespace {
 
 constexpr int kNT = 128;
-
-template <class T> const ModelDev<T>& dev_model(const HostModel& m);
-template <> const ModelDev<float>& dev_model<float>(const HostModel& m) { return m.dev32; }
-template <> const ModelDev<double>& dev_model<double>(const HostModel& m) { return m.dev64; }
 
 template <class T> struct DerivArgs {
   const T* q; const T* v; const T* vd;
@@ -147,31 +142,9 @@ __global__ void deriv_solve_kernel(const __grid_constant__ DerivDev D, const __g
   }
 }
 
-#define LAUNCH_CHECK(name) do { cudaError_t e_ = cudaGetLastError(); if (e_ != cudaSuccess) { rc = api_fail(RBD_ECUDA, std::string(name " launch failed: ") + cudaGetErrorString(e_)); goto done; } } while (0)
-
 // ---- model-specialised solve kernel (rbd_deriv_jit.cpp): compiled with NVRTC on the first large call (or ahead of time by
-// rbd_model_precompile_derivatives), cubin cached on disk, module cached per (tables, dtype, device) ----
-struct JitSolve {
-  int state = 0;                 // 1 = ready, -1 = unavailable (the generic kernel serves the call)
-  cudaLibrary_t lib = nullptr;
-  cudaKernel_t kernel = nullptr;
-  DerivJitPlan plan;
-  size_t smem = 0;
-  int bps = 0;
-};
-std::mutex g_jit_mu;
-std::map<std::string, JitSolve> g_jit;
+// rbd_model_precompile_derivatives), cubin cached on disk, loaded once per (precision, device) and owned by the handle ----
 
-bool jit_enabled() {
-  const char* e = std::getenv("RBD_JIT");
-  if (e && e[0] == '0') return false;
-  e = std::getenv("RBD_DERIV_JIT");
-  return !(e && e[0] == '0');
-}
-int64_t jit_min_batch() {
-  if (const char* e = std::getenv("RBD_JIT_MIN_BATCH")) return std::max<int64_t>(1, std::atoll(e));
-  return 4096;
-}
 // cubin for the model's solve kernel (from the cache, or compiled when `compile`); no GPU needed
 bool jit_solve_cubin(const DerivDev& D, const DerivAnc& A, bool f64, bool compile, DerivJitPlan& plan, std::vector<char>& cubin,
                      std::string& err) {
@@ -182,37 +155,35 @@ bool jit_solve_cubin(const DerivDev& D, const DerivAnc& A, bool f64, bool compil
   if (const char* dump = std::getenv("RBD_DERIV_DUMP")) {           // inspection: nvcc -cubin -Xptxas -v on the dumped text
     if (FILE* f = fopen((std::string(dump) + (f64 ? "_f64.cu" : "_f32.cu")).c_str(), "w")) { fwrite(src.data(), 1, src.size(), f); fclose(f); }
   }
-  bool from_cache = false;
-  return jit_compile_text(f64 ? "deriv_f64" : "deriv_f32", src, true, cubin, compile, &from_cache, err);
+  unsigned long long h = 1469598103934665603ull;            // FNV-1a of the text: the cache key
+  for (unsigned char c : src) { h ^= c; h *= 1099511628211ull; }
+  char name[64];
+  snprintf(name, sizeof name, "%016llx_deriv_%s", h, f64 ? "f64" : "f32");
+  return jit_cubin(name, true, compile, [&](std::string& s, std::string&) { s = std::move(src); return true; }, cubin, err);
 }
-JitSolve* jit_solve_get(const DerivDev& D, const DerivAnc& A, bool f64, int64_t B, const DeviceProps& p) {
-  if (!jit_enabled()) return nullptr;
-  std::string key((const char*)&D, sizeof(D));
-  key.append((const char*)A.anc, sizeof(int16_t) * D.nnz);
-  key.push_back(f64 ? 'd' : 'f');
-  key.push_back((char)p.dev);
-  std::lock_guard<std::mutex> lk(g_jit_mu);
-  JitSolve& e = g_jit[key];
+DerivSolve* jit_solve_get(rbd_model* m, const DerivDev& D, const DerivAnc& A, bool f64, int64_t B, const DeviceProps& p) {
+  const LaunchEnv& ev = launch_env();
+  std::lock_guard<std::mutex> lk(m->spec_mu);
+  DerivSolve& e = m->deriv[{f64, p.dev}];
   if (e.state == 1) return &e;
   if (e.state == -1) return nullptr;
+  DerivJitPlan plan;
   std::vector<char> cubin;
   std::string err;
-  if (!jit_solve_cubin(D, A, f64, B >= jit_min_batch(), e.plan, cubin, err)) {
+  if (!jit_solve_cubin(D, A, f64, B >= ev.deriv_jit_min_batch, plan, cubin, err)) {
     if (err != "no cached cubin") {
       e.state = -1;
-      if (std::getenv("RBD_JIT_VERBOSE")) fprintf(stderr, "rbd_b200: derivative solve kernel not specialised: %s\n", err.c_str());
+      if (ev.jit_verbose) fprintf(stderr, "rbd_b200: derivative solve kernel not specialised: %s\n", err.c_str());
     }
     return nullptr;
   }
+  e.warps = plan.warps;
   e.smem = (size_t)D.nnz * 32 * (f64 ? 8 : 4);
-  cudaError_t ce = cudaLibraryLoadData(&e.lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
-  if (ce == cudaSuccess) ce = cudaLibraryGetKernel(&e.kernel, e.lib, "rbd_deriv_solve");
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute((const void*)e.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e.smem);
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute((const void*)e.kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  if (ce == cudaSuccess) ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&e.bps, (const void*)e.kernel, 32 * e.plan.warps, e.smem);
+  cudaError_t ce = load_cubin(cubin, {{"rbd_deriv_solve", &e.kernel, e.smem, nullptr}}, e.lib);
+  if (ce == cudaSuccess) ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&e.bps, (const void*)e.kernel, 32 * e.warps, e.smem);
   if (ce != cudaSuccess || e.bps < 1) {
     cudaGetLastError();
-    if (std::getenv("RBD_JIT_VERBOSE")) fprintf(stderr, "rbd_b200: derivative solve kernel failed to load: %s\n", cudaGetErrorString(ce));
+    if (ev.jit_verbose) fprintf(stderr, "rbd_b200: derivative solve kernel failed to load: %s\n", cudaGetErrorString(ce));
     if (e.lib) { cudaLibraryUnload(e.lib); e.lib = nullptr; }
     e.state = -1;
     return nullptr;
@@ -221,9 +192,24 @@ JitSolve* jit_solve_get(const DerivDev& D, const DerivAnc& A, bool f64, int64_t 
   return &e;
 }
 
+// The last launch's error, else its geometry goes into the launch statistics.
+int launched(const char* name, int grid, int block, int smem_bytes, int blocks_per_sm) {
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return api_fail(RBD_ECUDA, std::string(name) + " launch failed: " + cudaGetErrorString(e));
+  api_note_launch(grid, block, smem_bytes, blocks_per_sm);
+  return RBD_OK;
+}
+
 template <class T>
 int derivatives_t(const rbd_model* model, int32_t dtype, int64_t B, int64_t ld, const T* q, const T* v, const T* tau, T* vd_out, T* dq,
                   T* dv, cudaStream_t stream) {
+  // read on every call, unlike the LaunchEnv switches: tests and tools change them while the process runs
+  const char* e_jit = std::getenv("RBD_DERIV_JIT");
+  const char* e_mb = std::getenv("RBD_DERIV_SCRATCH_MB");
+  const char* e_gf = std::getenv("RBD_DERIV_GLOBAL_FACTOR");
+  const bool jit = launch_env().jit && !(e_jit && e_jit[0] == '0');
+  const int64_t budget_mb = e_mb ? std::max<int64_t>(1, std::atoll(e_mb)) : 2048;
+  const bool global_factor = e_gf && e_gf[0] == '1';        // tests: exercise the fallback
   const HostModel& hm = model->hm;
   const ModelDev<T>& M = dev_model<T>(hm);
   DerivDev D;
@@ -234,8 +220,6 @@ int derivatives_t(const rbd_model* model, int32_t dtype, int64_t B, int64_t ld, 
   DeviceProps p;
   if (int rc = get_props(p)) return rc;
   // chunk size from the scratch budget
-  int64_t budget_mb = 2048;
-  if (const char* e = std::getenv("RBD_DERIV_SCRATCH_MB")) budget_mb = std::max<int64_t>(1, std::atoll(e));
   const int64_t per_sample = (int64_t)D.rows * (int64_t)sizeof(T);
   int64_t C = std::min<int64_t>(B, std::max<int64_t>(kNT, (budget_mb << 20) / per_sample / kNT * kNT));
   const int64_t sld = (C + 31) / 32 * 32;
@@ -244,7 +228,7 @@ int derivatives_t(const rbd_model* model, int32_t dtype, int64_t B, int64_t ld, 
     cudaGetLastError();
     return api_fail(RBD_ENOMEM, "rbd_dynamics_derivatives: scratch allocation failed (lower RBD_DERIV_SCRATCH_MB)");
   }
-  int rc = RBD_OK;
+  struct Guard { void* p; cudaStream_t s; ~Guard() { if (p) cudaFreeAsync(p, s); } } guard{scratch, stream};    // freed on every exit path
   // solve kernel geometry: warps per block so that factor + right-hand sides fit, maximising resident warps
   const size_t hbytes = (size_t)D.nnz * 32 * sizeof(T), xbytes = (size_t)D.nv * 32 * sizeof(T);
   int bestW = 0, bestNb = 0;
@@ -255,41 +239,37 @@ int derivatives_t(const rbd_model* model, int32_t dtype, int64_t B, int64_t ld, 
     const int W = (int)std::min<int64_t>(std::min(16, 2 * D.nv), avail / (int64_t)xbytes);
     if (W * nb > bestW * bestNb) { bestW = W; bestNb = nb; }
   }
-  if (const char* e = std::getenv("RBD_DERIV_GLOBAL_FACTOR")) { if (e[0] == '1') bestW = 0; }   // tests: exercise the fallback
+  if (global_factor) bestW = 0;
   if (bestW == 0) {       // factor too large for shared memory: read it from the scratch
     hs = false;
     bestW = (int)std::min<int64_t>(std::min(8, 2 * D.nv), p.max_smem_optin / (int64_t)xbytes);
     bestNb = 1;
   }
-  JitSolve* js = hs ? jit_solve_get(D, A, sizeof(T) == 8, B, p) : nullptr;
+  DerivSolve* js = hs && jit ? jit_solve_get(const_cast<rbd_model*>(model), D, A, sizeof(T) == 8, B, p) : nullptr;
   const size_t solve_smem = (hs ? hbytes : 0) + (size_t)bestW * xbytes;
   const size_t world_smem = (size_t)std::max(1, kin_rows(hm)) * kNT * sizeof(T);
   auto kworld = deriv_world_kernel<T, kNT>;
   auto ksolve_s = deriv_solve_kernel<T, true>;
   auto ksolve_g = deriv_solve_kernel<T, false>;
-  if ((rc = configure_once((const void*)kworld, p)) != RBD_OK) goto done;
-  if ((rc = configure_once(hs ? (const void*)ksolve_s : (const void*)ksolve_g, p)) != RBD_OK) goto done;
-  if (world_smem > (size_t)p.max_smem_optin) { rc = api_fail(RBD_EUNSUPPORTED, "rbd_dynamics_derivatives: too many open branch nodes"); goto done; }
+  if (int rc = configure_once((const void*)kworld, p)) return rc;
+  if (int rc = configure_once(hs ? (const void*)ksolve_s : (const void*)ksolve_g, p)) return rc;
+  if (world_smem > (size_t)p.max_smem_optin) return api_fail(RBD_EUNSUPPORTED, "rbd_dynamics_derivatives: too many open branch nodes");
   for (int64_t b0 = 0; b0 < B; b0 += C) {
     const int64_t c = std::min<int64_t>(C, B - b0);
     T* vd = vd_out + b0;
     // v̇ itself: the library's own forward dynamics (model-specialised kernels when available)
-    if ((rc = rbd_dynamics(model, dtype, c, ld, q + b0, v + b0, tau ? tau + b0 : nullptr, nullptr, vd, nullptr, stream)) != RBD_OK) goto done;
+    if (int rc = rbd_dynamics(model, dtype, c, ld, q + b0, v + b0, tau ? tau + b0 : nullptr, nullptr, vd, nullptr, stream)) return rc;
     DerivArgs<T> a{q + b0, v + b0, vd, dq + b0, dv + b0, scratch, ld, sld, c};
     const int gx = (int)((c + kNT - 1) / kNT);
     kworld<<<std::min(gx, 8 * p.sms), kNT, world_smem, stream>>>(M, D, a);
-    LAUNCH_CHECK("deriv_world_kernel");
-    api_note_launch(gx, kNT, (int)world_smem, 0);
+    if (int rc = launched("deriv_world_kernel", gx, kNT, (int)world_smem, 0)) return rc;
     deriv_accum_kernel<T, kNT><<<dim3(gx, kBodyRows), kNT, 0, stream>>>(M, D, a);
-    LAUNCH_CHECK("deriv_accum_kernel");
-    api_note_launch(gx * kBodyRows, kNT, 0, 0);
+    if (int rc = launched("deriv_accum_kernel", gx * kBodyRows, kNT, 0, 0)) return rc;
     deriv_pairs_kernel<T, kNT><<<dim3(D.nb, gx), kNT, 0, stream>>>(D, A, a);
-    LAUNCH_CHECK("deriv_pairs_kernel");
-    api_note_launch(gx * D.nb, kNT, 0, 0);
+    if (int rc = launched("deriv_pairs_kernel", gx * D.nb, kNT, 0, 0)) return rc;
     if (!hs) {
       deriv_factor_kernel<T, kNT><<<gx, kNT, 0, stream>>>(D, A, a);
-      LAUNCH_CHECK("deriv_factor_kernel");
-      api_note_launch(gx, kNT, 0, 0);
+      if (int rc = launched("deriv_factor_kernel", gx, kNT, 0, 0)) return rc;
     }
     if (js) {
       const T* Hg = scratch + (int64_t)D.h_base * sld;
@@ -297,22 +277,16 @@ int derivatives_t(const rbd_model* model, int32_t dtype, int64_t B, int64_t ld, 
       T* dq_ = dq + b0; T* dv_ = dv + b0;
       void* params[] = {(void*)&Hg, (void*)&sld_, (void*)&dq_, (void*)&dv_, (void*)&ld_, (void*)&c_};
       const int sgj = (int)std::min<int64_t>((c + 31) / 32, (int64_t)js->bps * p.sms);
-      if (cudaLaunchKernel((const void*)js->kernel, dim3(sgj), dim3(32 * js->plan.warps), params, js->smem, stream) != cudaSuccess) {
-        rc = api_fail(RBD_ECUDA, std::string("rbd_deriv_solve launch failed: ") + cudaGetErrorString(cudaGetLastError()));
-        goto done;
-      }
-      api_note_launch(sgj, 32 * js->plan.warps, (int)js->smem, js->bps);
+      cudaLaunchKernel((const void*)js->kernel, dim3(sgj), dim3(32 * js->warps), params, js->smem, stream);   // its error is also the last error
+      if (int rc = launched("rbd_deriv_solve", sgj, 32 * js->warps, (int)js->smem, js->bps)) return rc;
       continue;
     }
     const int sg = (int)std::min<int64_t>((c + 31) / 32, (int64_t)bestNb * p.sms);
     if (hs) ksolve_s<<<sg, dim3(32, bestW), solve_smem, stream>>>(D, A, a);
     else ksolve_g<<<sg, dim3(32, bestW), solve_smem, stream>>>(D, A, a);
-    LAUNCH_CHECK("deriv_solve_kernel");
-    api_note_launch(sg, 32 * bestW, (int)solve_smem, bestNb);
+    if (int rc = launched("deriv_solve_kernel", sg, 32 * bestW, (int)solve_smem, bestNb)) return rc;
   }
-done:
-  cudaFreeAsync(scratch, stream);
-  return rc;
+  return RBD_OK;
 }
 
 }  // namespace

@@ -4,9 +4,12 @@
 #include <cuda_runtime.h>
 
 #include <cstdlib>
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <string>
+#include <utility>
+#include <vector>
 
 #include "../../../include/rbd_b200.h"
 #include "rbd_codegen.h"
@@ -23,10 +26,19 @@ struct SpecEntry {
   int choice = 0;                // 0 = not tuned yet, 1 = kernel pair, 2 = unified CTA (for batches that fill the SMs)
   int uni_sw = 0;                // warps with a shared-memory stash in the unified CTA (0 = unified kernel unusable)
   int rows = 0;
-  bool from_cache = false;
   std::string why;               // reason for state -1
   int8_t kin_sign[kMaxBodies] = {0};   // SPEC_KIN: the path this entry was generated for
   bool kin_set = false;
+};
+
+// The model-specialised solve kernel of rbd_dynamics_derivatives (rbd_deriv.cu), loaded for one precision on one device.
+struct DerivSolve {
+  int state = 0;                 // 0 = not loaded yet, 1 = ready, -1 = unavailable (the table-driven solve kernel is used)
+  cudaLibrary_t lib = nullptr;
+  cudaKernel_t kernel = nullptr;
+  int warps = 0;                 // warps per CTA
+  size_t smem = 0;               // dynamic shared memory per CTA
+  int bps = 0;                   // resident CTAs per SM
 };
 
 constexpr int kCounterRing = 256;   // work-queue counters, one per call in flight
@@ -49,9 +61,10 @@ struct rbd_model {
   cudaEvent_t fork_ev[rbd::kEventRing] = {}, join_ev[rbd::kEventRing] = {};
   unsigned long long* counters = nullptr;     // [kCounterRing][2] device memory: work-queue counter, "needs generic kernel" flag
   unsigned next_call = 0;
-  // model-specialised kernels, keyed by SpecKey bits
+  // model-specialised kernels, keyed by SpecKey bits, and the derivatives' solve kernel, keyed by (fp64, device)
   std::mutex spec_mu;
   std::map<uint64_t, rbd::SpecEntry> spec;
+  std::map<std::pair<bool, int>, rbd::DerivSolve> deriv;
 };
 
 namespace rbd {
@@ -95,12 +108,21 @@ int spec_try_launch(rbd_model* m, const SpecKey& key, const SpecLaunchArgs& a, c
                     rbd_launch_info& li, const int** gate);
 // Compile (or load from the cubin cache) without launching; RBD_OK / RBD_EUNSUPPORTED.
 int spec_prepare(rbd_model* m, const SpecKey& key, bool load_on_device, std::string& err);
+// Unloads the handle's model-specialised kernels and derivative solve kernels.
 void spec_release(rbd_model* m);
+
+// One kernel of a cubin for load_cubin: its name, where its handle goes, the dynamic shared memory it is opted into (0: the
+// default) and, when `regs` is not NULL, where its registers per thread go.
+struct CubinKernel { const char* name; cudaKernel_t* kernel; size_t smem; int* regs; };
+// Loads `cubin`, looks up its kernels and gives each of them the largest shared-memory carve-out.  On failure the error is
+// cleared, nothing stays loaded and `lib` is NULL.
+cudaError_t load_cubin(const std::vector<char>& cubin, std::initializer_list<CubinKernel> kernels, cudaLibrary_t& lib);
 
 // Launch switches (DESIGN.md §4.7), read once per process.
 struct LaunchEnv {
   bool jit = true;                  // RBD_JIT=0: generic kernels only
   int64_t jit_min_batch = 1 << 15;  // below this a missing cubin is not compiled on the fly (generic kernels serve the call)
+  int64_t deriv_jit_min_batch = 4096;   // the same for rbd_dynamics_derivatives' solve kernel (RBD_JIT_MIN_BATCH sets both)
   int jit_variant = 0;              // RBD_JIT_VARIANT=1 (pair) / 2 (unified): skip the tuning
   bool jit_verbose = false;         // RBD_JIT_VERBOSE: print why a specialised kernel is unavailable
   bool no_tmem = false;             // RBD_NO_TMEM: single-kernel paths only
@@ -108,7 +130,10 @@ struct LaunchEnv {
   const char* only = nullptr;       // RBD_ONLY=smem|tmem: launch one kernel of a pair (ncu captures: the profiler serialises them)
   LaunchEnv() {
     if (const char* e = getenv("RBD_JIT")) jit = e[0] != '0';
-    if (const char* e = getenv("RBD_JIT_MIN_BATCH")) jit_min_batch = atoll(e);
+    if (const char* e = getenv("RBD_JIT_MIN_BATCH")) {
+      jit_min_batch = atoll(e);
+      deriv_jit_min_batch = jit_min_batch > 1 ? jit_min_batch : 1;
+    }
     if (const char* e = getenv("RBD_JIT_VARIANT")) jit_variant = atoi(e);
     jit_verbose = getenv("RBD_JIT_VERBOSE") != nullptr;
     no_tmem = getenv("RBD_NO_TMEM") != nullptr;

@@ -1,6 +1,5 @@
-// NVRTC front end + cubin cache for the model-specialised kernels (see rbd_jit.h).  Host-only C++.
+// NVRTC front end + cubin cache for the library's generated kernels (see rbd_jit.h).  Host-only C++.
 #include "rbd_jit.h"
-#include "rbd_jit_text.h"
 
 #include <dlfcn.h>
 #include <nvrtc.h>
@@ -55,14 +54,6 @@ Nvrtc& nvrtc() {
 bool dir_writable(const std::string& d) {
   mkdir(d.c_str(), 0755);
   return access(d.c_str(), W_OK | X_OK) == 0;
-}
-
-std::string key_name(const HostModel& hm, const SpecKey& k) {
-  char buf[96];
-  const char* algo = k.algo == SPEC_ABA ? "aba" : (k.algo == SPEC_RNEA ? "rnea" : (k.algo == SPEC_CRBA ? "crba" : "kin"));
-  snprintf(buf, sizeof buf, "%016llx_%s_%s_%d%d%d%s", (unsigned long long)spec_hash(hm, k), algo, k.f64 ? "f64" : "f32",
-           (int)k.has_in2, (int)k.has_out1, (int)k.lower, k.peers ? "p" : "");
-  return buf;
 }
 
 bool read_file(const std::string& path, std::vector<char>& out) {
@@ -138,37 +129,16 @@ static bool nvrtc_compile(const std::string& src, bool fmad, std::vector<char>& 
   return true;
 }
 
-bool jit_get_cubin(const HostModel& hm, const SpecKey& key, std::vector<char>& cubin, bool compile_if_missing, bool* from_cache,
-                   SpecStats* stats, std::string& err) {
-  const std::string path = jit_cache_dir() + "/" + key_name(hm, key) + ".cubin";
-  if (from_cache) *from_cache = false;
-  if (!getenv("RBD_JIT_NO_CACHE") && read_file(path, cubin)) {
-    if (from_cache) *from_cache = true;
-    return true;
-  }
+bool jit_cubin(const std::string& name, bool fmad, bool compile_if_missing,
+               const std::function<bool(std::string& src, std::string& err)>& source, std::vector<char>& cubin, std::string& err) {
+  const std::string path = jit_cache_dir() + "/" + name + ".cubin";
+  const bool use_cache = !getenv("RBD_JIT_NO_CACHE");
+  if (use_cache && read_file(path, cubin)) return true;
   if (!compile_if_missing) { err = "no cached cubin"; return false; }
   std::string src;
-  if (!spec_emit_cuda_tu(hm, key, src, stats, err)) return false;
-  if (!nvrtc_compile(src, false, cubin, err)) return false;
-  if (!getenv("RBD_JIT_NO_CACHE")) write_file_atomic(path, cubin.data(), cubin.size());
-  return true;
-}
-
-bool jit_compile_text(const std::string& tag, const std::string& src, bool fmad, std::vector<char>& cubin, bool compile_if_missing,
-                      bool* from_cache, std::string& err) {
-  unsigned long long h = 1469598103934665603ull;            // FNV-1a of the text: the cache key
-  for (unsigned char c : src) { h ^= c; h *= 1099511628211ull; }
-  char buf[64];
-  snprintf(buf, sizeof buf, "%016llx_%s", h, tag.c_str());
-  const std::string path = jit_cache_dir() + "/" + buf + ".cubin";
-  if (from_cache) *from_cache = false;
-  if (!getenv("RBD_JIT_NO_CACHE") && read_file(path, cubin)) {
-    if (from_cache) *from_cache = true;
-    return true;
-  }
-  if (!compile_if_missing) { err = "no cached cubin"; return false; }
+  if (!source(src, err)) return false;
   if (!nvrtc_compile(src, fmad, cubin, err)) return false;
-  if (!getenv("RBD_JIT_NO_CACHE")) write_file_atomic(path, cubin.data(), cubin.size());
+  if (use_cache) write_file_atomic(path, cubin.data(), cubin.size());
   return true;
 }
 

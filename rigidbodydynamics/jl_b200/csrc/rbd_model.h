@@ -25,6 +25,11 @@ struct HostModel {
   ModelDev<float> dev32;
 };
 
+// The device model in the kernels' scalar type.
+template <class T> const ModelDev<T>& dev_model(const HostModel& m);
+template <> inline const ModelDev<float>& dev_model<float>(const HostModel& m) { return m.dev32; }
+template <> inline const ModelDev<double>& dev_model<double>(const HostModel& m) { return m.dev64; }
+
 // Returns RBD_OK or an rbd_status; `err` gets a human-readable message.
 int build_host_model(const rbd_model_desc* desc, HostModel& out, std::string& err);
 

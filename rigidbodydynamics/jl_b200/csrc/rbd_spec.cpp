@@ -47,7 +47,38 @@ void spec_release(rbd_model* m) {
   std::lock_guard<std::mutex> lk(m->spec_mu);
   for (auto& kv : m->spec) if (kv.second.lib) cudaLibraryUnload(kv.second.lib);
   m->spec.clear();
+  for (auto& kv : m->deriv) if (kv.second.lib) cudaLibraryUnload(kv.second.lib);
+  m->deriv.clear();
 }
+
+cudaError_t load_cubin(const std::vector<char>& cubin, std::initializer_list<CubinKernel> kernels, cudaLibrary_t& lib) {
+  lib = nullptr;
+  cudaError_t e = cudaLibraryLoadData(&lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
+  for (const CubinKernel& k : kernels) {
+    if (e == cudaSuccess) e = cudaLibraryGetKernel(k.kernel, lib, k.name);
+    cudaFuncAttributes fa{};
+    if (e == cudaSuccess && k.regs) { e = cudaFuncGetAttributes(&fa, (const void*)*k.kernel); *k.regs = fa.numRegs; }
+    if (e == cudaSuccess && k.smem > 0) e = cudaFuncSetAttribute((const void*)*k.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute((const void*)*k.kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  }
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    if (lib) { cudaLibraryUnload(lib); lib = nullptr; }
+  }
+  return e;
+}
+
+namespace {
+// The cubin of (model, key), cached as <content hash>_<algo>_<f32|f64>_<flags>.cubin; the source is generated on a cache miss only.
+bool spec_cubin(const HostModel& hm, const SpecKey& k, bool compile_if_missing, std::vector<char>& cubin, std::string& err) {
+  char name[96];
+  const char* algo = k.algo == SPEC_ABA ? "aba" : (k.algo == SPEC_RNEA ? "rnea" : (k.algo == SPEC_CRBA ? "crba" : "kin"));
+  snprintf(name, sizeof name, "%016llx_%s_%s_%d%d%d%s", (unsigned long long)spec_hash(hm, k), algo, k.f64 ? "f64" : "f32",
+           (int)k.has_in2, (int)k.has_out1, (int)k.lower, k.peers ? "p" : "");
+  return jit_cubin(name, false, compile_if_missing,
+                   [&](std::string& src, std::string& e) { return spec_emit_cuda_tu(hm, k, src, nullptr, e); }, cubin, err);
+}
+}  // namespace
 
 // Straight-line programs far beyond the instruction caches run at the SM's instruction-fetch rate (~1.4 instr/clk on B200)
 // instead of its issue rate; measured against the generic (looping, cache-resident) kernels on Atlas: fp32 ABA 12.7 k nodes
@@ -67,36 +98,22 @@ int spec_prepare(rbd_model* m, const SpecKey& key, bool load_on_device, std::str
   if (se.state == 1) return RBD_OK;
   if (se.state == -1 && load_on_device) { err = se.why; return RBD_EUNSUPPORTED; }
   std::vector<char> cubin;
-  bool cached = false;
-  if (!jit_get_cubin(m->hm, key, cubin, true, &cached, nullptr, err)) {
+  if (!spec_cubin(m->hm, key, true, cubin, err)) {
     se.state = -1; se.why = err;
     return RBD_EUNSUPPORTED;
   }
   if (!load_on_device) return RBD_OK;      // precompile only (CPU build step): the cubin is in the cache now
-  cudaError_t e = cudaLibraryLoadData(&se.lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
-  if (e == cudaSuccess) e = cudaLibraryGetKernel(&se.k_smem, se.lib, "rbd_jit_smem");
-  if (e == cudaSuccess) e = cudaLibraryGetKernel(&se.k_tmem, se.lib, "rbd_jit_tmem");
-  if (e == cudaSuccess) e = cudaLibraryGetKernel(&se.k_uni, se.lib, "rbd_jit_uni");
-  cudaFuncAttributes fa{};
-  if (e == cudaSuccess) { e = cudaFuncGetAttributes(&fa, (const void*)se.k_smem); se.regs_smem = fa.numRegs; }
-  if (e == cudaSuccess) { e = cudaFuncGetAttributes(&fa, (const void*)se.k_tmem); se.regs_tmem = fa.numRegs; }
-  if (e == cudaSuccess) { e = cudaFuncGetAttributes(&fa, (const void*)se.k_uni); se.regs_uni = fa.numRegs; }
-  if (e == cudaSuccess) e = cudaFuncSetAttribute((const void*)se.k_tmem, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   se.rows = spec_stash_rows(m->hm, key);
   const size_t smem = (size_t)std::max(1, se.rows) * 32 * (key.f64 ? 8 : 4);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute((const void*)se.k_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute((const void*)se.k_smem, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   se.uni_sw = spec_uni_smem_warps(m->hm, key);
-  if (e == cudaSuccess && se.uni_sw > 0) e = cudaFuncSetAttribute((const void*)se.k_uni, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem * se.uni_sw));
-  if (e == cudaSuccess) e = cudaFuncSetAttribute((const void*)se.k_uni, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  const cudaError_t e = load_cubin(cubin, {{"rbd_jit_smem", &se.k_smem, smem, &se.regs_smem},
+                                           {"rbd_jit_tmem", &se.k_tmem, 0, &se.regs_tmem},
+                                           {"rbd_jit_uni", &se.k_uni, se.uni_sw > 0 ? smem * se.uni_sw : 0, &se.regs_uni}}, se.lib);
   if (e != cudaSuccess) {
-    cudaGetLastError();
     se.state = -1;
     se.why = err = std::string("loading the specialised cubin: ") + cudaGetErrorString(e);
-    if (se.lib) { cudaLibraryUnload(se.lib); se.lib = nullptr; }
     return RBD_EUNSUPPORTED;
   }
-  se.from_cache = cached;
   se.state = 1;
   return RBD_OK;
 }
@@ -130,8 +147,7 @@ int spec_try_launch(rbd_model* m, const SpecKey& key, const SpecLaunchArgs& a, c
     if (a.B < ev.jit_min_batch) {          // small call and nothing loaded yet: use a cached cubin if there is one, never compile
       std::vector<char> probe;
       std::string e2;
-      bool cached = false;
-      if (!jit_get_cubin(m->hm, key, probe, false, &cached, nullptr, e2)) return RBD_OK;
+      if (!spec_cubin(m->hm, key, false, probe, e2)) return RBD_OK;
     }
     std::string e2;
     if (spec_prepare(m, key, true, e2) != RBD_OK) {      // generic kernels take over; the reason is kept in the entry
